@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W             (N > 1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR
 
 A "step" registers the BASELINE.json configs[2] batch: --pairs-total (default 4096) consecutive scan pairs (64 rings x
 2048 azimuth steps = 131 072 points per scan, 75 x 24 spherical voxels, 7 iterations, X0 = 0), pair-sharded by contiguous
@@ -12,7 +13,8 @@ HBM when the timed region starts (`value`), or start in pinned host memory (`e2e
 measures what the host->device link of this box sustains with all ranks copying at once).  `configs` holds the other
 BASELINE.json configurations (latency of one 64-channel pair, the 128-channel pair, scan-to-submap at 2 M points).
 
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  --dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (see
+dump_outputs): the inputs are a pure function of the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -28,6 +30,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: bench.py writes nothing into it
 
 RINGS, AZIM = 64, 2048
 NPTS = RINGS * AZIM
@@ -37,6 +40,8 @@ METRIC = "registrations/s (64-ch, 75x24 vox, 7 it)"
 README_PAIRS_PER_S = 1000.0 / 35.0  # reference README.md:59: 35 ms / pair on a Ryzen 5800X (other hardware)
 B_ALG_PER_PAIR = 12 * (NPTS + NPTS) + 192  # SURVEY.md 8(d)
 DEFAULT_CHUNK = 512  # pairs per launch of the device-resident batch (the library's default, icet_b200_set_chunk)
+DUMP_LIMIT = 64_000_000  # bytes of all --dump-outputs files together (64 MB)
+NPY_HEADER_MAX = 4096  # allowance per .npy file for its header (numpy writes 128 bytes for these arrays)
 
 
 def peaks():
@@ -170,7 +175,7 @@ def run_reference(args, rank: int, world: int):
     # one step = `sample` pairs: 2 per host thread (bounded so that the whole run ends within minutes)
     sample = max(2, min(2 * cores, 256))
     scans = synth_host.scans(sample + 1, first_scan=0, seed=SEED, rings=RINGS, azim=AZIM)
-    cb, _ = cpu_baseline_measure(scans, cores, warmup=max(1, args.warmup), steps=max(1, args.steps))
+    cb, _ = cpu_baseline_measure(scans, cores, warmup=max(1, args.warmup), steps=args.steps)
     value = cb["value"]
     t = sample / value
     total, per_gpu, scaling = resolve_pairs(args, world)
@@ -324,6 +329,27 @@ def bench_configs(ctx, stream, dev, latency):
     return out
 
 
+def dump_outputs(out_dir: str, rows: np.ndarray, recs: np.ndarray) -> None:
+    """--dump-outputs: the results of every pair of the last timed step, one DIR/<name>.npy per field.
+    rows: [N, 48] float32, what a step returns (X | pred_stds | Q, in global pair order); recs: [N, 5] float32 words,
+    the remaining fields of the same result records (status, n_gauss1, n_used, n_dropped as int32 bits, cond).
+    Integer fields are written as float64 (exact).  When the files would exceed DUMP_LIMIT bytes, a fixed seeded
+    sample of the pairs is written; pair_index.npy always names the pairs that were."""
+    n = rows.shape[0]
+    ints = np.ascontiguousarray(recs[:, :4]).view(np.int32).astype(np.float64)
+    arrays = {"X": rows[:, 0:6], "pred_stds": rows[:, 6:12], "Q": rows[:, 12:48].reshape(n, 6, 6),
+              "status": ints[:, 0], "n_gauss1": ints[:, 1], "n_used": ints[:, 2], "n_dropped": ints[:, 3],
+              "cond": recs[:, 4], "pair_index": np.arange(n, dtype=np.float64)}
+    per_pair = sum(a.nbytes for a in arrays.values()) // max(1, n)
+    budget = DUMP_LIMIT - NPY_HEADER_MAX * len(arrays)
+    if per_pair * n > budget:
+        keep = np.sort(np.random.default_rng(SEED).choice(n, budget // per_pair, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -344,7 +370,13 @@ def main():
     ap.add_argument("--host-chunk", type=int, default=0, help="pairs per chunk of the host-buffer pipeline (0 = default)")
     ap.add_argument("--unfused", action="store_true", help="diagnostic: 3 launches per iteration instead of k_loop")
     ap.add_argument("--persistent", action="store_true", help="diagnostic: the persistent loop kernel for every chunk")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (GPU path only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
 
@@ -417,10 +449,14 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(stream)
     for _ in range(args.steps):
-        step()
+        rows = step()
     ev1.record(stream)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:  # before anything below reuses `results`
+        recs = sharding.gather_results(results[:, 48:53], world)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, rows.cpu().numpy(), recs.cpu().numpy())
     launches = ctx.kernel_launches - l0
     t_ms = ev0.elapsed_time(ev1)
     tt = torch.tensor([t_ms, float(launches)], dtype=torch.float64, device=dev)
@@ -490,7 +526,7 @@ def main():
             e2e_step()
         barrier()
         t0 = time.perf_counter()
-        nst = max(2, args.steps)
+        nst = args.steps
         for _ in range(nst):
             e2e_step()
         barrier()

@@ -6,9 +6,9 @@ bench.py's cpu_baseline / reference arm -- never from the icet_b200 package.
 from __future__ import annotations
 
 import ctypes as C
-import hashlib
 import os
 import subprocess
+import tempfile
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -68,23 +68,24 @@ class _Out(C.Structure):
                 [("evec1_in", _FP), ("evec1_in_mask", _BP), ("X_in", _FP)])
 
 
-def _build(native: bool) -> str:
+def _build() -> str:
     """Compile the oracle if the .so is missing or older than its sources."""
-    if native:
-        # -march=native objects must be built on the machine that runs them
-        with open("/proc/cpuinfo") as f:
-            flags = next((l for l in f if l.startswith("flags")), "")
-        tag = hashlib.sha1(flags.encode()).hexdigest()[:10]
-        out = os.path.join(_HERE, "_build", "native-" + tag)
-        target, goal = os.path.join(out, "libicet_oracle_native.so"), "native"
-    else:
-        out = os.path.join(_HERE, "_build")
-        target, goal = os.path.join(out, "libicet_oracle.so"), "all"
+    out = os.path.join(_HERE, "_build")
+    target = os.path.join(out, "libicet_oracle.so")
     srcs = [os.path.join(_HERE, f) for f in ("icet_oracle.cpp", "icet_oracle.h", "eigen_algos.h", "Makefile")]
     if (not os.path.exists(target)) or os.path.getmtime(target) < max(map(os.path.getmtime, srcs)):
-        subprocess.run(["make", "-C", _HERE, goal, "OUT=" + out], check=True,
+        subprocess.run(["make", "-C", _HERE, "all", "OUT=" + out], check=True,
                        stdout=subprocess.DEVNULL)
     return target
+
+
+def _load_native() -> C.CDLL:
+    """-march=native code must be built on the machine that runs it, so it is built at run time, once per process, in
+    a private temporary directory: the source tree is never written (it may be read-only) and no other build is
+    ever picked up.  The library stays mapped after the directory is removed."""
+    with tempfile.TemporaryDirectory(prefix="icet_oracle_native-") as out:
+        subprocess.run(["make", "-C", _HERE, "native", "OUT=" + out], check=True, stdout=subprocess.DEVNULL)
+        return C.CDLL(os.path.join(out, "libicet_oracle_native.so"))
 
 
 _LIBS: dict = {}
@@ -92,7 +93,7 @@ _LIBS: dict = {}
 
 def lib(native: bool = False) -> C.CDLL:
     if native not in _LIBS:
-        L = C.CDLL(_build(native))
+        L = _load_native() if native else C.CDLL(_build())
         L.icet_oracle_run.restype = C.c_int
         L.icet_oracle_run.argtypes = [C.POINTER(_Params), _FP, C.c_int32, C.c_int32, _FP, C.c_int32,
                                       C.c_int32, _FP, C.POINTER(_Out)]

@@ -1011,3 +1011,32 @@ def test_against_reference_build(ctx, po, parity, name):
     parity.add("gpu_vs_reference_build", name, gaussians=int(has.sum()), dX_m=dm, dX_rad=dr, sign_unstable_voxels=nflip,
                bounds_cnt1_has1_bit_identical=True)
     print("%s: GPU vs the reference build: |dX| %.1e m %.1e rad, %d Gaussians, %d sign-unstable" % (name, dm, dr, has.sum(), nflip))
+
+
+def test_bench_dump_outputs(ctx, tmp_path):
+    """bench.py --steps K times K steps (the kernel launches of the timed window scale with K), and --dump-outputs
+    writes what its last timed step computed: the result records of the synthetic sequence, bit-identical to a direct
+    call on the same scans."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from conftest import ROOT
+    pairs = 8
+    ref = register_sequence(ctx, synth_device(ctx, pairs + 1))
+    launches = {}
+    for steps in (1, 2):
+        out = tmp_path / ("steps%d" % steps)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3",
+                            "--pairs-total", str(pairs), "--no-configs", "--no-cpu-baseline", "--no-latency", "--no-e2e",
+                            "--no-callers", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps
+        launches[steps] = line["gpu_launches"]
+        d = {f[:-4]: np.load(out / f) for f in os.listdir(out)}
+        assert all(a.dtype in (np.float32, np.float64) and a.shape[0] == pairs for a in d.values())
+        np.testing.assert_array_equal(d["pair_index"], np.arange(pairs))
+        for name in ("X", "pred_stds", "Q", "status", "n_gauss1", "n_used", "n_dropped", "cond"):
+            np.testing.assert_array_equal(d[name], ref[name], err_msg=name)
+    assert launches[1] > 0 and launches[2] == 2 * launches[1], launches

@@ -153,6 +153,47 @@ def test_bench_reference_arm_runs():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["higher_is_better"] is True
 
 
+def test_bench_dump_outputs_layout(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float32 / float64 .npy per field of the result records (integer fields exact);
+    above the size cap, the same seeded sample of the pairs on every run, named by pair_index."""
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)   # importing bench.py sets it
+    import bench
+    n = 50
+    rows = np.random.default_rng(1).standard_normal((n, 48)).astype(np.float32)
+    recs = np.random.default_rng(2).standard_normal((n, 5)).astype(np.float32)
+    ints = np.arange(4 * n, dtype=np.int32).reshape(n, 4)
+    recs[:, :4] = ints.view(np.float32)
+
+    def load(d):
+        return {f[:-4]: np.load(d / f) for f in os.listdir(d)}
+
+    bench.dump_outputs(str(tmp_path / "all"), rows, recs)
+    d = load(tmp_path / "all")
+    assert sorted(d) == sorted(["X", "pred_stds", "Q", "status", "n_gauss1", "n_used", "n_dropped", "cond", "pair_index"])
+    assert all(a.dtype in (np.float32, np.float64) and a.shape[0] == n for a in d.values())
+    np.testing.assert_array_equal(d["X"], rows[:, :6])
+    np.testing.assert_array_equal(d["Q"].reshape(n, 36), rows[:, 12:])
+    np.testing.assert_array_equal(d["n_used"], ints[:, 2])
+    np.testing.assert_array_equal(d["cond"], recs[:, 4])
+    per_pair = sum(a.nbytes for a in d.values()) // n
+    limit = 20 * per_pair + bench.NPY_HEADER_MAX * len(d)
+    monkeypatch.setattr(bench, "DUMP_LIMIT", limit)
+    for k in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / k), rows, recs)
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    idx = a["pair_index"].astype(np.int64)
+    assert len(idx) == 20 and np.all(np.diff(idx) > 0)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= limit
+    for name in a:
+        np.testing.assert_array_equal(a[name], b[name])
+        np.testing.assert_array_equal(a[name], d[name][idx])
+
+
+def test_bench_rejects_zero_steps():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def _build_demo():
     r = subprocess.run(["make", "-C", os.path.join(ROOT, "examples")], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr

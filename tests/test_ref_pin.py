@@ -66,7 +66,9 @@ def test_oracle_reproduces_reference_golden(po, name):
     s1, s2 = _inputs(name, g)
     rl, nphi, nth = (int(v) for v in g["params"])
     mode = int(g["order_mode"])
-    o = po.run(s1, s2, X0=g["x0"], dumps="small", order_mode=mode, runlen=rl, bins_phi=nphi, bins_theta=nth)
+    ntb = g["n_thresh_buff"] if "n_thresh_buff" in g else (25, 0.1, 0.1)
+    o = po.run(s1, s2, X0=g["x0"], dumps="small", order_mode=mode, runlen=rl, bins_phi=nphi, bins_theta=nth,
+               n=int(ntb[0]), thresh=float(ntb[1]), buff=float(ntb[2]))
     _check(name, g, o, shipped=(mode == po.ORDER_REF_SHIPPED))
 
 

@@ -40,6 +40,13 @@ def cases():
         out.append((name + "_presorted", presort(s1), s2, None, po.ORDER_SORTED, {}))
     d = np.load(os.path.join(GOLDEN, "inputs_frame.npz"))
     out.append(("frame_shipped_x0demo", d["scan1"], d["scan2"], [1, 0, 0, 0, 0, 0], po.ORDER_REF_SHIPPED, {}))
+    # the other settings test_live_reference_build_matches_oracle reruns the reference with
+    out.append(("frame_shipped_x0tilt", d["scan1"], d["scan2"], [-0.3, 0.2, 0.0, 0.01, 0.0, -0.02], po.ORDER_REF_SHIPPED,
+                {}))
+    out.append(("frame_presorted_loose", presort(d["scan1"]), d["scan2"], None, po.ORDER_SORTED,
+                dict(n=40, thresh=0.3, buff=0.5)))
+    out.append(("frame_presorted_coarse", presort(d["scan1"]), d["scan2"], None, po.ORDER_SORTED,
+                dict(runlen=3, bins_phi=12, bins_theta=40)))
     sc = synth_host.scans(2, first_scan=100)
     out.append(("synth100_shipped", sc[0], sc[1], None, po.ORDER_REF_SHIPPED, {}))
     out.append(("synth100_presorted", presort(sc[0]), sc[1], None, po.ORDER_SORTED, {}))
@@ -106,6 +113,7 @@ def main():
                                 x0=np.zeros(6, np.float32) if x0 is None else np.float32(x0), order_mode=mode,
                                 eigen="shim" if a.eigen_include is None else a.eigen_include,
                                 params=np.int32([kw.get("runlen", 7), kw.get("bins_phi", 24), kw.get("bins_theta", 75)]),
+                                n_thresh_buff=np.float32([kw.get("n", 25), kw.get("thresh", 0.1), kw.get("buff", 0.1)]),
                                 n_ellipsoids=ref["n_ellipsoids"], **{k: ref[k] for k in KEYS}, **extra)
     print("oracle == reference build:", "YES" if ok else "NO")
     return 0 if ok else 1
