@@ -4,9 +4,9 @@ Python host-side mirror of the reference interface (`class ICET`, reference incl
 over the C ABI of include/icet_b200.h.  There is no CPU fallback: importing works anywhere, but
 every compute entry point raises if the CUDA library or a B200 is missing.
 """
-from .api import ICET, Context, IcetError, MultiContext, Params, Result, lib_path, load_library  # noqa: F401
+from .api import ICET, Context, IcetError, Keyframe, MultiContext, Params, Result, lib_path, load_library  # noqa: F401
 from .build import build  # noqa: F401
 from .nodes import MapMakerNode, Node, OdometryNode, PointMap, ScanMatcherNode  # noqa: F401
 
-__all__ = ["ICET", "Context", "MultiContext", "IcetError", "Params", "Result", "build", "load_library", "lib_path",
+__all__ = ["ICET", "Context", "Keyframe", "MultiContext", "IcetError", "Params", "Result", "build", "load_library", "lib_path",
            "OdometryNode", "MapMakerNode", "ScanMatcherNode", "Node", "PointMap"]

@@ -3,6 +3,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import weakref
 from dataclasses import dataclass
 
 import numpy as np
@@ -119,7 +120,9 @@ EXPORTS = ["icet_b200_version", "icet_b200_last_error", "icet_b200_create", "ice
            "icet_b200_transform_cloud_device", "icet_b200_transform_cloud",
            "icet_b200_multi_create", "icet_b200_multi_destroy", "icet_b200_multi_devices", "icet_b200_multi_context",
            "icet_b200_register_batch_multi", "icet_b200_register_sequence_multi_device", "icet_b200_multi_gathered",
-           "icet_b200_multi_gathered_host"]
+           "icet_b200_multi_gathered_host", "icet_b200_keyframe_create", "icet_b200_keyframe_create_device",
+           "icet_b200_keyframe_destroy", "icet_b200_keyframe_gaussians", "icet_b200_register_keyframe",
+           "icet_b200_register_keyframe_batch_device"]
 NKERNELS = 11
 
 _LIB = None
@@ -196,6 +199,12 @@ def load_library() -> C.CDLL:
     L.icet_b200_register_sequence_multi_device.argtypes = [vp, C.POINTER(Params), C.c_int32, vp, C.c_int32]
     L.icet_b200_multi_gathered.argtypes = [vp, C.c_int32, C.POINTER(vp), C.POINTER(C.c_int32)]
     L.icet_b200_multi_gathered_host.argtypes = [vp, C.c_int32, vp]
+    L.icet_b200_keyframe_create.argtypes = [vp, C.POINTER(Params), vp, C.c_int32, C.c_int32, C.POINTER(vp)]
+    L.icet_b200_keyframe_create_device.argtypes = [vp, C.POINTER(Params), vp, C.c_int32, C.c_int32, C.POINTER(vp)]
+    L.icet_b200_keyframe_destroy.argtypes = [vp]
+    L.icet_b200_keyframe_gaussians.argtypes = [vp]
+    L.icet_b200_register_keyframe.argtypes = [vp, C.POINTER(Params), vp, C.c_int32, C.c_int32, vp, C.POINTER(Result)]
+    L.icet_b200_register_keyframe_batch_device.argtypes = [vp, C.POINTER(Params), C.c_int32, vp, vp, vp, vp]
     _LIB = L
     return L
 
@@ -224,6 +233,7 @@ class Context:
         self._L = load_library()
         h = C.c_void_p()
         self._h = None
+        self._keyframes = weakref.WeakSet()  # closed before the context: they live in its device memory
         self._check(self._L.icet_b200_create(device, C.byref(h)))
         self._h = h
 
@@ -234,6 +244,8 @@ class Context:
 
     def close(self):
         if self._h is not None:
+            for kf in list(self._keyframes):
+                kf.close()
             self._L.icet_b200_destroy(self._h)
             self._h = None
 
@@ -521,3 +533,93 @@ class ICET:
         self.Q = r["Q"].copy()
         self.status = int(r["status"])
         self.result = r
+
+
+class Keyframe:
+    """Scan 1 fitted once (icet_b200_keyframe_create): register any number of scans against it without refitting it --
+    a scan against an accumulated map, one pair from several initial guesses, scans k+1 .. k+m against keyframe k.
+    Results are bit-identical to `Context.register(scan1, scan2, ...)` with the same settings.
+
+        kf = Keyframe(map_points)                       # N x 3 or [3, N] host cloud
+        r = kf.register(scan, X0)                       # one RESULT_DTYPE record
+        kf.register_batch_device(ptrs2, n2, out_ptr)    # device scans, asynchronous
+
+    The bins, n, thresh, buff and the row-order mode are those of the keyframe; runlen and the loop / scan-2 flags are
+    chosen per call."""
+
+    def __init__(self, scan1, num_bins_phi=24, num_bins_theta=75, n=25, thresh=0.1, buff=0.1, ctx: Context | None = None,
+                 shipped_row_order=False, _device=None):
+        self._h = None
+        self._ctx = ctx or default_context()
+        self._L = self._ctx._L
+        self.shipped_row_order = bool(shipped_row_order)
+        self._p = make_params(0, num_bins_phi, num_bins_theta, n, thresh, buff,
+                              flags=FLAG_SHIPPED_ORDER if shipped_row_order else 0)
+        h = C.c_void_p()
+        if _device is None:
+            s1 = as_planes(scan1)
+            rc = self._L.icet_b200_keyframe_create(self._ctx._h, C.byref(self._p), s1.ctypes.data, s1.shape[1],
+                                                   s1.shape[1], C.byref(h))
+        else:
+            ptr, n1, ld1 = _device
+            rc = self._L.icet_b200_keyframe_create_device(self._ctx._h, C.byref(self._p), C.c_void_p(ptr), n1, ld1,
+                                                          C.byref(h))
+        self._ctx._check(rc)
+        self._h = h
+        self._ctx._keyframes.add(self)
+
+    @classmethod
+    def from_device(cls, ptr: int, n1: int, ld1: int | None = None, **kw) -> "Keyframe":
+        """scan 1 as float32 planes in DEVICE memory (leading dimension ld1, default n1)."""
+        return cls(None, _device=(ptr, n1, n1 if ld1 is None else ld1), **kw)
+
+    def _handle(self):
+        if self._h is None:
+            raise IcetError("keyframe is closed")
+        return self._h
+
+    def params(self, runlen=7, flags=0) -> Params:
+        """icet_b200_params of a registration against this keyframe."""
+        p = make_params(runlen, self._p.bins_phi, self._p.bins_theta, self._p.n, self._p.thresh, self._p.buff, flags)
+        p.flags |= self._p.flags
+        return p
+
+    @property
+    def n_gauss1(self) -> int:
+        h = self._handle()
+        return self._ctx._check(self._L.icet_b200_keyframe_gaussians(h))
+
+    def register(self, scan2, X0=None, runlen=7, flags=0):
+        """One HOST scan 2 against the keyframe (blocking); returns one RESULT_DTYPE record."""
+        h = self._handle()
+        p = self.params(runlen, flags)
+        s2 = as_planes(scan2)
+        x0 = np.zeros(6, np.float32) if X0 is None else np.ascontiguousarray(X0, np.float32)
+        res = Result()
+        self._ctx._check(self._L.icet_b200_register_keyframe(h, C.byref(p), s2.ctypes.data, s2.shape[1], s2.shape[1],
+                                                             x0.ctypes.data, C.byref(res)))
+        return np.frombuffer(bytes(res), dtype=RESULT_DTYPE)[0]
+
+    def register_batch_device(self, ptrs2, n2, out_ptr: int, x0_ptr: int = 0, runlen=7, flags=0):
+        """DEVICE scans ptrs2[i] (n2[i] points each) against the keyframe; x0 (npairs x 6 or 0) and out (npairs
+        records) in DEVICE memory.  Asynchronous on the context's stream."""
+        h = self._handle()
+        p = self.params(runlen, flags)
+        a2 = ptrs2 if isinstance(ptrs2, np.ndarray) else np.array(ptrs2, np.uint64)
+        assert a2.dtype == np.uint64 and a2.flags["C_CONTIGUOUS"]
+        n2 = np.ascontiguousarray(n2, np.int32)
+        assert n2.shape == a2.shape
+        self._ctx._check(self._L.icet_b200_register_keyframe_batch_device(
+            h, C.byref(p), len(a2), a2.ctypes.data, n2.ctypes.data, C.c_void_p(x0_ptr) if x0_ptr else None,
+            C.c_void_p(out_ptr)))
+
+    def close(self):
+        if self._h is not None:
+            self._L.icet_b200_keyframe_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

@@ -176,6 +176,8 @@ int icet_b200_set_lanes(icet_b200_ctx* c, int32_t n) {
 
 int64_t icet_b200_kernel_launches(icet_b200_ctx* c) { return c ? c->launches : 0; }
 
+// (k_kf_attach, the scan-1 set-up of a keyframe chunk, is counted under id 1: it does k_cell_scan's per-pair
+// initialisation)
 static const char* const k_names[ICET_B200_NKERNELS] = {"k_scan1_bin", "k_cell_scan", "k_scatter", "k_cluster",
                                                         "k_pass<scan1>", "k_fit1", "k_prep2", "k_pass<scan2>",
                                                         "k_vox2", "k_solve6", "k_loop"};
@@ -224,10 +226,11 @@ int icet_b200_set_dump(icet_b200_ctx* c, int32_t enable) {
 // -- device-resident batch --------------------------------------------------------------------
 static int batch_device_impl(icet_b200_ctx* c, const icet_b200_params* p, int32_t npairs, const PairDesc* h_desc,
                              const float* d_x0, icet_b200_result* d_out, bool dump, const PairDesc* d_desc_all = nullptr,
-                             int nmax_dev = 0) {
+                             int nmax_dev = 0, const icet_b200_keyframe* kf = nullptr) {
   // h_desc lives in host memory; descriptors are uploaded per chunk through the pinned bounce buffer.
   // d_desc_all (callers layer): the descriptors are already on the device -- built there, with data-dependent
   // sizes no larger than nmax_dev -- and h_desc is not read.
+  // kf: scan 1 of every pair is this keyframe (the descriptors hold no scan 1).
   int rc = ensure_pinned(c, (size_t)std::min(npairs, c->chunk_pairs) * sizeof(PairDesc) * ICET_NLANE + 4096);
   if (rc) return rc;
   // consecutive chunks alternate between the two compute lanes (own stream + workspace each); lane 1 starts after
@@ -275,7 +278,7 @@ static int batch_device_impl(icet_b200_ctx* c, const icet_b200_params* p, int32_
     }
     const float* x0c = d_x0 ? d_x0 + (chain ? 0 : (size_t)base * 6) : nullptr;
     if (chain && base > 0) x0c = d_out[base - 1].X;  // stream order: the previous chunk has finished by then
-    rc = run_chunk(c, p, P, d_desc, n1max, n2max, x0c, d_out + base, dump, lane);
+    rc = run_chunk(c, p, P, d_desc, n1max, n2max, x0c, d_out + base, dump, lane, kf);
     if (rc) return rc;
   }
   for (int l = 1; l < nl; l++) {
@@ -502,6 +505,189 @@ int icet_b200_register(icet_b200_ctx* c, const icet_b200_params* p, const float*
   const float* pa = a.data();
   const float* pb = b.data();
   return icet_b200_register_batch(c, p, 1, &pa, &n1, &pb, &n2, x0, out);
+}
+
+// -- keyframes -----------------------------------------------------------------------------------
+// A registration's params must describe the keyframe's scan-1 fit.
+static int keyframe_params(const icet_b200_keyframe* kf, const icet_b200_params* p) {
+  if (!kf) return fail(ICET_B200_E_INVALID, "keyframe is NULL");
+  int rc = validate(p);
+  if (rc) return rc;
+  const icet_b200_params& k = kf->p;
+  if (p->bins_phi != k.bins_phi) return fail(ICET_B200_E_INVALID, "bins_phi differs from the keyframe's");
+  if (p->bins_theta != k.bins_theta) return fail(ICET_B200_E_INVALID, "bins_theta differs from the keyframe's");
+  if (p->n != k.n) return fail(ICET_B200_E_INVALID, "n differs from the keyframe's");
+  if (p->thresh != k.thresh) return fail(ICET_B200_E_INVALID, "thresh differs from the keyframe's");
+  if (p->buff != k.buff) return fail(ICET_B200_E_INVALID, "buff differs from the keyframe's");
+  if ((p->flags ^ k.flags) & ICET_B200_FLAG_SHIPPED_ORDER)
+    return fail(ICET_B200_E_INVALID, "ICET_B200_FLAG_SHIPPED_ORDER differs from the keyframe's");
+  if (p->flags & ICET_B200_FLAG_CHAIN_X0)
+    return fail(ICET_B200_E_INVALID, "ICET_B200_FLAG_CHAIN_X0 is not supported against a keyframe");
+  return 0;
+}
+
+// Copies a HOST cloud (planes, leading dimension ld) into n-strided DEVICE planes at dst.
+static int upload_planes(icet_b200_ctx* c, float* dst, const float* src, int32_t n, int32_t ld) {
+  if (n == 0) return 0;
+  if (ld == n) {
+    CK(cudaMemcpyAsync(dst, src, (size_t)3 * n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    return 0;
+  }
+  for (int k = 0; k < 3; k++)
+    CK(cudaMemcpyAsync(dst + (size_t)k * n, src + (size_t)k * ld, (size_t)n * sizeof(float), cudaMemcpyHostToDevice,
+                       c->stream));
+  return 0;
+}
+
+int icet_b200_keyframe_create_device(icet_b200_ctx* c, const icet_b200_params* p, const float* scan1, int32_t n1,
+                                     int32_t ld1, icet_b200_keyframe** out) {
+  if (!c) return fail(ICET_B200_E_INVALID, "ctx is NULL");
+  if (!out) return fail(ICET_B200_E_INVALID, "keyframe out-pointer is NULL");
+  *out = nullptr;
+  int rc = validate(p);
+  if (rc) return rc;
+  if (n1 < 0 || ld1 < n1 || (n1 > 0 && !scan1)) return fail(ICET_B200_E_INVALID, "bad scan1 / n1 / ld1");
+  CK(cudaSetDevice(c->device));
+  // the scan-1 set-up of one pair without scan 2 or iterations (it also starts the pair's result record)
+  icet_b200_params q = *p;
+  q.runlen = 0;
+  q.flags = p->flags & ICET_B200_FLAG_SHIPPED_ORDER;
+  rc = ensure_pinned(c, 4096);
+  if (rc) return rc;
+  rc = c->descbuf[0].ensure(sizeof(PairDesc));
+  if (rc) return rc;
+  rc = c->resbuf.ensure(sizeof(icet_b200_result));
+  if (rc) return rc;
+  CK(cudaStreamSynchronize(c->stream));  // the pinned bounce buffer may still feed an earlier upload
+  PairDesc* hd = (PairDesc*)c->pinned;
+  *hd = PairDesc{scan1, nullptr, n1, ld1, 0, 0};
+  CK(cudaMemcpyAsync(c->descbuf[0].p, hd, sizeof(PairDesc), cudaMemcpyHostToDevice, c->stream));
+  icet_b200_result* d_res = (icet_b200_result*)c->resbuf.p;
+  ChunkRun r;
+  rc = chunk_setup(c, &q, 1, (const PairDesc*)c->descbuf[0].p, n1, 0, nullptr, d_res, false, 0, r);
+  if (!rc) rc = chunk_scan1(r);
+  c->last_valid = false;  // lane 0's workspace now holds this chunk
+  if (rc) return rc;
+  CK(cudaGetLastError());
+  icet_b200_keyframe* kf = new icet_b200_keyframe();
+  kf->ctx = c;
+  kf->p = q;
+  const size_t ncell = (size_t)p->bins_phi * p->bins_theta;
+  rc = kf->rec.ensure(ncell * sizeof(CellRec));
+  if (!rc) rc = kf->vox.ensure(ncell * sizeof(Vox1));
+  if (rc) {
+    icet_b200_keyframe_destroy(kf);
+    return rc;
+  }
+  int32_t* h_ng = (int32_t*)((char*)c->pinned + 1024);
+  cudaError_t e = cudaMemcpyAsync(kf->rec.p, r.ck.rec, ncell * sizeof(CellRec), cudaMemcpyDeviceToDevice, c->stream);
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(kf->vox.p, r.ck.vox, ncell * sizeof(Vox1), cudaMemcpyDeviceToDevice, c->stream);
+  if (e == cudaSuccess)
+    e = cudaMemcpyAsync(h_ng, &d_res->n_gauss1, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  if (e != cudaSuccess) {
+    icet_b200_keyframe_destroy(kf);
+    return fail(ICET_B200_E_CUDA, std::string("keyframe copy: ") + cudaGetErrorString(e));
+  }
+  kf->n_gauss1 = *h_ng;
+  *out = kf;
+  return 0;
+}
+
+int icet_b200_keyframe_create(icet_b200_ctx* c, const icet_b200_params* p, const float* scan1, int32_t n1, int32_t ld1,
+                              icet_b200_keyframe** out) {
+  if (!c) return fail(ICET_B200_E_INVALID, "ctx is NULL");
+  if (!out) return fail(ICET_B200_E_INVALID, "keyframe out-pointer is NULL");
+  *out = nullptr;
+  int rc = validate(p);
+  if (rc) return rc;
+  if (n1 < 0 || ld1 < n1 || (n1 > 0 && !scan1)) return fail(ICET_B200_E_INVALID, "bad scan1 / n1 / ld1");
+  CK(cudaSetDevice(c->device));
+  CK(cudaEventSynchronize(c->ev_done[0]));
+  rc = c->stage[0].ensure(std::max<size_t>(1, (size_t)3 * n1) * sizeof(float));
+  if (rc) return rc;
+  float* d_s1 = (float*)c->stage[0].p;
+  rc = upload_planes(c, d_s1, scan1, n1, ld1);
+  if (rc) return rc;
+  return icet_b200_keyframe_create_device(c, p, d_s1, n1, n1, out);
+}
+
+int icet_b200_keyframe_destroy(icet_b200_keyframe* kf) {
+  if (!kf) return 0;
+  icet_b200_ctx* c = kf->ctx;
+  cudaSetDevice(c->device);
+  cudaStreamSynchronize(c->stream);
+  for (int l = 1; l < ICET_NLANE; l++)
+    if (c->lanes[l]) cudaStreamSynchronize(c->lanes[l]);
+  kf->rec.release();
+  kf->vox.release();
+  delete kf;
+  return 0;
+}
+
+int icet_b200_keyframe_gaussians(icet_b200_keyframe* kf) {
+  if (!kf) return fail(ICET_B200_E_INVALID, "keyframe is NULL");
+  return kf->n_gauss1;
+}
+
+int icet_b200_register_keyframe(icet_b200_keyframe* kf, const icet_b200_params* p, const float* scan2, int32_t n2,
+                                int32_t ld2, const float x0[6], icet_b200_result* out) {
+  int rc = keyframe_params(kf, p);
+  if (rc) return rc;
+  if (!out) return fail(ICET_B200_E_INVALID, "out is NULL");
+  if (n2 < 0 || ld2 < n2 || (n2 > 0 && !scan2)) return fail(ICET_B200_E_INVALID, "bad scan2 / n2 / ld2");
+  icet_b200_ctx* c = kf->ctx;
+  CK(cudaSetDevice(c->device));
+  CK(cudaEventSynchronize(c->ev_done[0]));
+  rc = c->stage[0].ensure(std::max<size_t>(1, (size_t)3 * n2) * sizeof(float));
+  if (rc) return rc;
+  rc = c->descbuf[0].ensure(sizeof(PairDesc));
+  if (rc) return rc;
+  rc = c->x0buf[0].ensure(6 * sizeof(float));
+  if (rc) return rc;
+  rc = c->resbuf.ensure(sizeof(icet_b200_result));
+  if (rc) return rc;
+  rc = ensure_pinned(c, 4096);
+  if (rc) return rc;
+  CK(cudaStreamSynchronize(c->stream));  // the pinned bounce buffer may still feed an earlier upload
+  float* d_s2 = (float*)c->stage[0].p;
+  rc = upload_planes(c, d_s2, scan2, n2, ld2);
+  if (rc) return rc;
+  PairDesc* hd = (PairDesc*)c->pinned;
+  *hd = PairDesc{nullptr, d_s2, 0, 0, n2, n2};
+  CK(cudaMemcpyAsync(c->descbuf[0].p, hd, sizeof(PairDesc), cudaMemcpyHostToDevice, c->stream));
+  const float* d_x0 = nullptr;
+  if (x0) {
+    float* hx = (float*)((char*)c->pinned + 256);
+    memcpy(hx, x0, 6 * sizeof(float));
+    CK(cudaMemcpyAsync(c->x0buf[0].p, hx, 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    d_x0 = (const float*)c->x0buf[0].p;
+  }
+  icet_b200_result* d_res = (icet_b200_result*)c->resbuf.p;
+  rc = run_chunk(c, p, 1, (const PairDesc*)c->descbuf[0].p, 0, n2, d_x0, d_res, false, 0, kf);
+  if (rc) return rc;
+  CK(cudaMemcpyAsync(out, d_res, sizeof(icet_b200_result), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return check_loop_watchdog(c);
+}
+
+int icet_b200_register_keyframe_batch_device(icet_b200_keyframe* kf, const icet_b200_params* p, int32_t npairs,
+                                             const float* const* scan2, const int32_t* n2, const float* x0,
+                                             icet_b200_result* out) {
+  int rc = keyframe_params(kf, p);
+  if (rc) return rc;
+  if (npairs < 0 || (npairs > 0 && (!scan2 || !n2 || !out))) return fail(ICET_B200_E_INVALID, "NULL argument");
+  if (npairs == 0) return 0;
+  icet_b200_ctx* c = kf->ctx;
+  CK(cudaSetDevice(c->device));
+  std::vector<PairDesc> d(npairs);
+  for (int i = 0; i < npairs; i++) {
+    if (n2[i] < 0 || (n2[i] > 0 && !scan2[i]))
+      return fail(ICET_B200_E_INVALID, "bad scan pointer / size in pair " + std::to_string(i));
+    d[i] = PairDesc{nullptr, scan2[i], 0, 0, n2[i], n2[i]};
+  }
+  return batch_device_impl(c, p, npairs, d.data(), x0, out, false, nullptr, 0, kf);
 }
 
 int icet_b200_get_dump(icet_b200_ctx* c, icet_b200_voxel_dump* o) {

@@ -465,6 +465,41 @@ __global__ void __launch_bounds__(128) k_fit1(const Chunk ck) {
 }
 
 // ----------------------------------------------------------------------------------------------
+// Keyframe chunks (icet_b200_register_keyframe*): K1-K4 ran once, when the keyframe was created, and left its CellRec /
+// Vox1 records (after k_fit1) in krec / kvox.  This kernel puts them into the slots of every pair of the chunk, anchors
+// the scan-2 frames of the active voxels at R(X0) with the chunk's fs2 as k_fit1 does, and starts the pair like
+// k_cell_scan.  After it the scan-2 kernels see the same state as after k_fit1.  Grid: (ceil(ncell / 128), P).
+// ----------------------------------------------------------------------------------------------
+static_assert(sizeof(CellRec) == 32 && sizeof(Vox1) % 8 == 0, "k_kf_attach copies CellRec as 2 float4, Vox1 as 8-byte words");
+__global__ void __launch_bounds__(128) k_kf_attach(const Chunk ck, const CellRec* __restrict__ krec,
+                                                   const Vox1* __restrict__ kvox, int n_gauss1) {
+  pdl_prologue();
+  __shared__ float s_tr[12];
+  const int pair = blockIdx.y;
+  pair_start(ck, pair, n_gauss1, s_tr, blockIdx.x == 0);
+  const int c0 = blockIdx.x * 128, nc = min(128, ck.ncell - c0);
+  const size_t pc = (size_t)pair * ck.ncell + c0;
+  {  // flat copies of the block's cells, consecutive threads on consecutive words
+    const uint2* vs = reinterpret_cast<const uint2*>(kvox + c0);
+    uint2* vd = reinterpret_cast<uint2*>(ck.vox + pc);
+    for (int w = threadIdx.x; w < nc * (int)(sizeof(Vox1) / 8); w += 128) vd[w] = __ldg(vs + w);
+    const float4* rs = reinterpret_cast<const float4*>(krec + c0);
+    float4* rd = reinterpret_cast<float4*>(ck.rec + pc);
+    for (int w = threadIdx.x; w < 2 * nc; w += 128) rd[w] = __ldg(rs + w);
+  }
+  __syncthreads();  // s_tr
+  if ((int)threadIdx.x < nc) {
+    const float4* rp = reinterpret_cast<const float4*>(krec + c0 + threadIdx.x);
+    const float4 ra = __ldg(rp);
+    if (__float_as_uint(ra.z) & F_ACTIVE2) {
+      float ax, ay, az, sc;
+      vox_anchor2_rec(ra, __ldg(rp + 1), s_tr, ck.fs2, ax, ay, az, sc);
+      ck.anch[pc + threadIdx.x] = make_float4(ax, ay, az, sc);
+    }
+  }
+}
+
+// ----------------------------------------------------------------------------------------------
 // prepScan2 (src/icet.cpp:254-277): points2_OG = sphericalToCartesian(cartesianToSpherical(scan2)).
 // (The radial re-ordering of scan 2 only changes the reference's summation order.)
 // ----------------------------------------------------------------------------------------------

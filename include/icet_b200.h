@@ -164,6 +164,39 @@ int icet_b200_synchronize(icet_b200_ctx* ctx);
  * (0 = default 8; a batch uses at most one lane per 512-pair chunk, batches below 4096 pairs at most four). */
 int icet_b200_set_lanes(icet_b200_ctx* ctx, int32_t lanes);
 
+/* -- keyframes ---------------------------------------------------------------------------------------------------------
+ * Many registrations often share their scan 1: a scan against an accumulated map (scan-to-map localisation), one pair
+ * from several initial guesses, scans k+1 .. k+m against keyframe k.  The scan-1 half of the reference's constructor
+ * (fitScan1, src/icet.cpp:68-107) depends only on scan 1 and the bin parameters, so a keyframe runs it once and keeps
+ * its result (cluster bounds, Gaussians, L / U of every voxel) on the device; registrations against it start from there.
+ * Results are bit-identical to registering the same pairs with the cloud as scan 1.
+ * A keyframe belongs to the context that created it and, like the context, is not thread-safe; destroy it before the
+ * context.  Keyframe registrations record no per-voxel dump and, like batches, end the get_points2 / classify_scan2
+ * record of the last icet_b200_register call. */
+typedef struct icet_b200_keyframe icet_b200_keyframe; /* scan-1 state of one cloud, resident on the ctx's device */
+
+/* fitScan1 once.  p: bins_phi, bins_theta, n, thresh, buff and ICET_B200_FLAG_SHIPPED_ORDER are fixed for the keyframe;
+ * runlen and the other flags are ignored.  HOST planes (leading dimension ld1), blocking. */
+int icet_b200_keyframe_create(icet_b200_ctx* ctx, const icet_b200_params* p, const float* scan1, int32_t n1,
+                              int32_t ld1, icet_b200_keyframe** kf);
+/* Same, scan1 in DEVICE memory (e.g. a map from icet_b200_map_get_device with a host-known count).  Blocking. */
+int icet_b200_keyframe_create_device(icet_b200_ctx* ctx, const icet_b200_params* p, const float* scan1, int32_t n1,
+                                     int32_t ld1, icet_b200_keyframe** kf);
+int icet_b200_keyframe_destroy(icet_b200_keyframe* kf);   /* synchronises the ctx's stream first */
+int icet_b200_keyframe_gaussians(icet_b200_keyframe* kf); /* = result.n_gauss1 of every registration against it */
+
+/* The registrations below require p to agree with the keyframe in bins_phi, bins_theta, n, thresh, buff and
+ * ICET_B200_FLAG_SHIPPED_ORDER, and reject ICET_B200_FLAG_CHAIN_X0 (ICET_B200_E_INVALID).  runlen and the loop / scan-2
+ * flags apply per call, as in a batch. */
+/* icet_b200_register with scan 1 = the keyframe.  HOST scan 2, blocking. */
+int icet_b200_register_keyframe(icet_b200_keyframe* kf, const icet_b200_params* p, const float* scan2, int32_t n2,
+                                int32_t ld2, const float x0[6], icet_b200_result* out);
+/* icet_b200_register_batch_device with scan1[i] = the keyframe for every i: scan2[i] DEVICE pointers (host table),
+ * x0 (npairs*6 or NULL) and out DEVICE memory, asynchronous on the ctx's stream. */
+int icet_b200_register_keyframe_batch_device(icet_b200_keyframe* kf, const icet_b200_params* p, int32_t npairs,
+                                             const float* const* scan2, const int32_t* n2, const float* x0,
+                                             icet_b200_result* out);
+
 /* -- per-voxel state of the most recent single-pair call (icet_b200_register) ------------------
  * Mirrors the public members the reference exposes for visualisation / debugging:
  *   clusterBounds (include/icet.h:83), sigma1/mu1/L/U (:89-94), pointIndices sizes (:95-96).
