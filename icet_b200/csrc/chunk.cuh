@@ -15,7 +15,7 @@ int fail(int code, const std::string& msg) {
   } while (0)
 
 constexpr int FPB = 21;                 // fixed-point basis: CellRec::scale maps the voxel's box diameter D to 2^(FPB-1)
-constexpr int FP_LIM = (1 << FPB);      // (the per-chunk multipliers Chunk::fs1 / fs2 refine it, see fp_bits in runtime.inl)
+constexpr int FP_LIM = (1 << FPB);      // (the per-pair multiplier FixPt::fs refines it, see fp_bits below)
 constexpr unsigned FULL = 0xffffffffu;
 constexpr uint32_t F_STAT1 = 1u;        // scan-1 statistics wanted for this cell
 constexpr uint32_t F_ACTIVE2 = 2u;      // voxel takes part in the scan-2 loop
@@ -38,6 +38,35 @@ struct PairDesc {
   const float* s2;
   int n1, ld1, n2, ld2;
 };
+
+// Fixed-point refinement of the per-voxel accumulators of a cloud of n points: offsets are quantised to
+// round(d * CellRec::scale * fs), clamped to +-fl, with fs = 2^(bits - FPB) and fl = 2^bits.  Offsets up to 2^bits,
+// products up to 2^(2 bits), 64-bit sums over at most n points: 2 bits + ceil(log2 n) <= 62.  As fine as that allows
+// (131 072 points: 2^22 levels per box diameter, i.e. ~2 um at 50 m -- below the fp32 ulp of the coordinates
+// themselves).  A function of the pair's own cloud (PairDesc::n1 for scan 1, n2 for scan 2), never of the other pairs
+// of its chunk: the result of a pair does not depend on how a batch is cut into chunks or ordered.
+__host__ __device__ __forceinline__ int fp_bits(int n) {
+  const unsigned m = (unsigned)(n > 2 ? n : 2) - 1u;  // ceil(log2(max(n, 2))) = bit length of m
+#ifdef __CUDA_ARCH__
+  const int lg = 32 - __clz(m);
+#else
+  const int lg = 32 - __builtin_clz(m);
+#endif
+  const int b = (62 - lg) / 2;
+  return b < 12 ? 12 : (b > 23 ? 23 : b);
+}
+struct FixPt {
+  float fs;  // multiplier of CellRec::scale (a power of two)
+  int fl;    // clamp of the offsets
+};
+__host__ __device__ __forceinline__ FixPt fix_point(int n) {
+  const int b = fp_bits(n);
+#ifdef __CUDA_ARCH__
+  return FixPt{__int_as_float((127 + b - FPB) << 23), 1 << b};
+#else
+  return FixPt{ldexpf(1.0f, b - FPB), 1 << b};
+#endif
+}
 
 struct __align__(16) CellRec {  // read by the pass kernels: first half by every point, second half per run of inside points
   float inner, outer;           // clusterBounds columns 4,5 (src/icet.cpp:149)
@@ -80,12 +109,7 @@ struct Chunk {  // everything a kernel needs, passed by value
   const PairDesc* desc;
   int npairs, ncell, nT, nP, n, runlen, flags;
   float thresh, buff;
-  int n1max, n2max;
-  // fixed-point refinement per scan: offsets are quantised to round(d * CellRec::scale * fs), clamped to +-fl.  As fine
-  // as 64-bit sums of products allow for the chunk's largest cloud (131 072 points: 2^22 levels per box diameter, i.e.
-  // ~2 um at 50 m -- below the fp32 ulp of the coordinates themselves)
-  float fs1, fs2;
-  int fl1, fl2;
+  int n1max, n2max;  // capacities of the per-pair arrays below (the fixed-point precision of a pair: fix_point)
   // scan 1
   int32_t* cellid1;  // [P][n1max]
   float* r1;         // [P][n1max]

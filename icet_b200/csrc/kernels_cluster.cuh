@@ -204,12 +204,13 @@ __global__ void __launch_bounds__(CL_THREADS, 1) k_loop_cluster(const Chunk ck, 
                                   recs, tr, md, pair, __ldg(ck.nz2 + pair));
         } else {
           unsigned long long* accp = ck.acc + (size_t)pair * ck.ncell * NQ;
+          const int n2 = __ldg(&ck.desc[pair].n2);
           for (int tile = gwarp; tile < tiles; tile += nwarp)
             pass_warp_tile<true, CL_K, 2, 4>(ck, went, tab, recs, tr, ck.pog + (size_t)pair * 3 * ck.n2max,
-                                             (size_t)ck.n2max, n, tile * 32 * CL_K, accp);
+                                             (size_t)ck.n2max, n, tile * 32 * CL_K, fix_point(n2), accp);
           if (gwarp == nwarp - 1 && lane == 0)
             pass_dropped_returns(ck, reinterpret_cast<const float4*>(tab), reinterpret_cast<const float4*>(tab) + ck.nT + 2,
-                                 recs, tr, accp, __ldg(ck.nz2 + pair));
+                                 recs, tr, accp, __ldg(ck.nz2 + pair), n2);
         }
       }
       if (share) {  // (uniform) the helpers' tiles before the voxel phase

@@ -97,7 +97,7 @@ __device__ __forceinline__ void vox_algebra(const Chunk& ck, int pair, int cell,
 #pragma unroll
   for (int k = 0; k < NQ; k++) qp[k] = 0ull;
   double mean[3], cov[6];
-  stats_from_acc(q, rc, ck.fs2, mean, cov);
+  stats_from_acc(q, rc, fix_point(__ldg(&ck.desc[pair].n2)).fs, mean, cov);
   vox_algebra_core(ck, pair, cell, iter, Jm, (long long)q[0], mean, cov, acc);
 }
 
@@ -200,7 +200,7 @@ __device__ __forceinline__ void load_vox_mode(const Chunk& ck, int pair, VoxMode
   const int2 h = __ldcg(reinterpret_cast<const int2*>(pm));
   vm.set = h.x;
   vm.rebuild = h.y;
-  vm.fs2 = ck.fs2;
+  vm.fs2 = fix_point(__ldg(&ck.desc[pair].n2)).fs;
   const float4* tb = reinterpret_cast<const float4*>(pm->TRb);
   const float4* tp = reinterpret_cast<const float4*>(ck.TR + (size_t)pair * 12);
 #pragma unroll
@@ -847,11 +847,12 @@ __global__ void __launch_bounds__(PASS_THREADS, 3) k_loop(const Chunk ck, int ti
             pass2_dropped_returns(ck, reinterpret_cast<const float4*>(tab), reinterpret_cast<const float4*>(tab) + ck.nT + 2,
                                   recs, tr, md, pair, __ldg(ck.nz2 + pair));
         } else {
+        const int n2 = __ldg(&ck.desc[pair].n2);
         pass_warp_tile<true, K, 2, (K <= 4 ? K : 1)>(ck, went, tab, recs, tr, ck.pog + (size_t)pair * 3 * ck.n2max, (size_t)ck.n2max, n, w0,
-                                accp, (ck.dump_on && iter == 3 && tile < 2048) ? ck.dump.tl + (size_t)ck.runlen * 16 + 4096 + tile : nullptr);
+                                fix_point(n2), accp, (ck.dump_on && iter == 3 && tile < 2048) ? ck.dump.tl + (size_t)ck.runlen * 16 + 4096 + tile : nullptr);
         if (tile == 0 && lane == 0)
           pass_dropped_returns(ck, reinterpret_cast<const float4*>(tab), reinterpret_cast<const float4*>(tab) + ck.nT + 2,
-                               recs, tr, accp, __ldg(ck.nz2 + pair));
+                               recs, tr, accp, __ldg(ck.nz2 + pair), n2);
         }
         if (tile == 0) TL(7);
         if (ck.dump_on && iter == 3 && tile < 2048 && lane == 0) ck.dump.tl[(size_t)ck.runlen * 16 + 2 * tile + 1] = gtime();

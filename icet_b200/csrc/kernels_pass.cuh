@@ -73,7 +73,7 @@ __device__ __forceinline__ void point_stage2(float r, float th, float ph, float 
 // The dropped returns of scan 2: points2_OG == (0,0,0) for all of them, so they all land on t * R
 // (src/icet.cpp:377-378; SURVEY.md A.12) -- evaluated once per iteration, weighted with their number.
 __device__ inline void pass_dropped_returns(const Chunk& ck, const float4* tth, const float4* tph, const CellRec* recs,
-                                            const float* tr, unsigned long long* accp, long long nz) {
+                                            const float* tr, unsigned long long* accp, long long nz, int n2) {
   if (nz <= 0) return;
   int c;
   bool active, in;
@@ -84,8 +84,9 @@ __device__ inline void pass_dropped_returns(const Chunk& ck, const float4* tth, 
   red_add(q, (unsigned long long)nz);
   if (in) {
     const CellRec rc = recs[c];
+    const FixPt fp = fix_point(n2);
     int ix, iy, iz;
-    point_stage2(r, th, ph, rc.refx, rc.refy, rc.refz, rc.scale * ck.fs2, ck.fl2, ix, iy, iz);
+    point_stage2(r, th, ph, rc.refx, rc.refy, rc.refz, rc.scale * fp.fs, fp.fl, ix, iy, iz);
     const long long fx = ix, fy = iy, fz = iz;
     red_add(q + 1, (unsigned long long)nz);
     red_add(q + 2, (unsigned long long)(nz * fx));
@@ -132,7 +133,7 @@ __device__ __forceinline__ void flush_in_run(unsigned long long* accp, int cell,
 template <bool SCAN2, int K, int PF = 2, int G = 1>
 __device__ __forceinline__ void pass_warp_tile(const Chunk& ck, int4* went /* the warp's pass_wslots(K) slots */,
                                                const float* tab, const CellRec* recs, const float* tr,
-                                               const float* px_, size_t ld, int n, int w0,
+                                               const float* px_, size_t ld, int n, int w0, FixPt fp,
                                                unsigned long long* accp, unsigned long long* dbg_stamp = nullptr,
                                                const int32_t* s1_cell = nullptr, const float* s1_th = nullptr,
                                                const float* s1_ph = nullptr) {
@@ -279,11 +280,10 @@ __device__ __forceinline__ void pass_warp_tile(const Chunk& ck, int4* went /* th
       pxx = pxy = pxz = pyy = pyz = pzz = 0;
       const float4* rp = reinterpret_cast<const float4*>(recs + cur);
       const float4 ra = __ldg(rp), rb = __ldg(rp + 1);
-      sc = ra.w * (SCAN2 ? ck.fs2 : ck.fs1); refx = rb.x; refy = rb.y; refz = rb.z;
+      sc = ra.w * fp.fs; refx = rb.x; refy = rb.y; refz = rb.z;
     }
     int fx, fy, fz;
-    point_stage2(__int_as_float(v.y), __int_as_float(v.z), __int_as_float(v.w), refx, refy, refz, sc,
-                 SCAN2 ? ck.fl2 : ck.fl1, fx, fy, fz);
+    point_stage2(__int_as_float(v.y), __int_as_float(v.z), __int_as_float(v.w), refx, refy, refz, sc, fp.fl, fx, fy, fz);
     nin++;
     sx += fx; sy += fy; sz += fz;
     pxx += (long long)fx * fx; pxy += (long long)fx * fy; pxz += (long long)fx * fz;
@@ -347,12 +347,12 @@ __global__ void __launch_bounds__(PASS_THREADS, MINB) k_pass(const Chunk ck) {
   unsigned long long* accp = ck.acc + (size_t)pair * ck.ncell * NQ;
   __syncthreads();
   pass_warp_tile<SCAN2, K, PF, G>(ck, ent + (threadIdx.x >> 5) * pass_wslots(K), tab, recs, tr, px_, ld, n,
-                           tile0 + (threadIdx.x >> 5) * 32 * K, accp, nullptr,
+                           tile0 + (threadIdx.x >> 5) * 32 * K, fix_point(SCAN2 ? d.n2 : d.n1), accp, nullptr,
                            SCAN2 ? nullptr : (grouped ? ck.cellg : ck.cellid1) + o1,
                            SCAN2 ? nullptr : (grouped ? ck.thg : ck.th1) + o1, SCAN2 ? nullptr : (grouped ? ck.phg : ck.ph1) + o1);
   if (SCAN2 && blockIdx.x == 0 && threadIdx.x == 0)
     pass_dropped_returns(ck, reinterpret_cast<const float4*>(tab), reinterpret_cast<const float4*>(tab) + ck.nT + 2, recs, tr,
-                         accp, ck.nz2[pair]);
+                         accp, ck.nz2[pair], d.n2);
 }
 
 // exact-sum -> mean / covariance (double) of a voxel
@@ -389,6 +389,7 @@ __global__ void __launch_bounds__(128) k_fit1(const Chunk ck) {
   const size_t ci = (size_t)pair * ck.ncell + cell;
   CellRec rc = ck.rec[ci];
   unsigned long long* q = ck.acc + ci * NQ;
+  const PairDesc d = ck.desc[pair];
   bool has = false;
   if (rc.flags & F_STAT1) {
     const long long nin = (long long)q[1];
@@ -397,7 +398,7 @@ __global__ void __launch_bounds__(128) k_fit1(const Chunk ck) {
     if (3 * nin >= ck.n && nin >= 2) {
       has = true;
       double mean[3], cov[6];
-      stats_from_acc(q, rc, ck.fs1, mean, cov);
+      stats_from_acc(q, rc, fix_point(d.n1).fs, mean, cov);
       Vox1 v;
       for (int k = 0; k < 3; k++) v.mu[k] = mean[k];
       const double d1 = (double)(rc.cnt1 - 1);  // `indices1.size() - 1` (:315)
@@ -456,7 +457,7 @@ __global__ void __launch_bounds__(128) k_fit1(const Chunk ck) {
     float trb[12], ax, ay, az, sc;
     for (int k = 0; k < 12; k++) trb[k] = ck.pm[pair].TRb[k];
     vox_anchor2_rec(make_float4(rc.inner, rc.outer, __uint_as_float(fl), rc.scale),
-                    make_float4(rc.refx, rc.refy, rc.refz, __int_as_float(rc.cnt1)), trb, ck.fs2, ax, ay, az, sc);
+                    make_float4(rc.refx, rc.refy, rc.refz, __int_as_float(rc.cnt1)), trb, fix_point(d.n2).fs, ax, ay, az, sc);
     ck.anch[ci] = make_float4(ax, ay, az, sc);
   }
   if (rc.flags & F_STAT1)
@@ -467,7 +468,7 @@ __global__ void __launch_bounds__(128) k_fit1(const Chunk ck) {
 // ----------------------------------------------------------------------------------------------
 // Keyframe chunks (icet_b200_register_keyframe*): K1-K4 ran once, when the keyframe was created, and left its CellRec /
 // Vox1 records (after k_fit1) in krec / kvox.  This kernel puts them into the slots of every pair of the chunk, anchors
-// the scan-2 frames of the active voxels at R(X0) with the chunk's fs2 as k_fit1 does, and starts the pair like
+// the scan-2 frames of the active voxels at R(X0) with the pair's fixed-point scale as k_fit1 does, and starts the pair like
 // k_cell_scan.  After it the scan-2 kernels see the same state as after k_fit1.  Grid: (ceil(ncell / 128), P).
 // ----------------------------------------------------------------------------------------------
 static_assert(sizeof(CellRec) == 32 && sizeof(Vox1) % 8 == 0, "k_kf_attach copies CellRec as 2 float4, Vox1 as 8-byte words");
@@ -493,7 +494,7 @@ __global__ void __launch_bounds__(128) k_kf_attach(const Chunk ck, const CellRec
     const float4 ra = __ldg(rp);
     if (__float_as_uint(ra.z) & F_ACTIVE2) {
       float ax, ay, az, sc;
-      vox_anchor2_rec(ra, __ldg(rp + 1), s_tr, ck.fs2, ax, ay, az, sc);
+      vox_anchor2_rec(ra, __ldg(rp + 1), s_tr, fix_point(ck.desc[pair].n2).fs, ax, ay, az, sc);
       ck.anch[pc + threadIdx.x] = make_float4(ax, ay, az, sc);
     }
   }

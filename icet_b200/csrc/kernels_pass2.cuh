@@ -36,7 +36,7 @@ constexpr float INC_MAX_SA = 1.0e-3f;         // sum |dR|_F   (x 30 m = 3 cm)
 constexpr float INC_MAX_SB = 0.05f;           // sum |dt|     (metres)
 // (The members of a voxel sit within one box diameter D of its anchor when they are evaluated and the anchor drifts by
 // at most r * INC_MAX_SA + INC_MAX_SB < D (D >= 0.2 r + 0.2 m) before the next rebuild re-anchors it: the +-2 D range of
-// the fixed-point frame (Chunk::fl2) is never left.)
+// the fixed-point frame (FixPt::fl) is never left.)
 
 struct Pass2Mode {  // block-uniform copy of the pair's PairMode + accumulator set
   bool rebuild;
@@ -223,12 +223,13 @@ __device__ __forceinline__ void vox_anchor2_rec(float4 ra, float4 rb, const floa
 __device__ __forceinline__ void anchors_update(const Chunk& ck, int pair, const float* trb, int tid, int nth) {
   const CellRec* recs = ck.rec + (size_t)pair * ck.ncell;
   float4* an = ck.anch + (size_t)pair * ck.ncell;
+  const float fs2 = fix_point(ck.desc[pair].n2).fs;
   for (int c = tid; c < ck.ncell; c += nth) {
     const float4* rp = reinterpret_cast<const float4*>(recs + c);
     const float4 ra = __ldcg(rp);
     if (!(__float_as_uint(ra.z) & F_ACTIVE2)) continue;
     float ax, ay, az, sc;
-    vox_anchor2_rec(ra, __ldcg(rp + 1), trb, ck.fs2, ax, ay, az, sc);
+    vox_anchor2_rec(ra, __ldcg(rp + 1), trb, fs2, ax, ay, az, sc);
     an[c] = make_float4(ax, ay, az, sc);
   }
 }
@@ -499,8 +500,9 @@ __device__ __forceinline__ void load_pass2_mode(const Chunk& ck, int pair, Pass2
   const int4 h = __ldcg(reinterpret_cast<const int4*>(pm));             // set, rebuild, SA, C
   md.rebuild = h.y != 0;
   md.set = h.x;
-  md.fs2 = ck.fs2;
-  md.fl2 = ck.fl2;
+  const FixPt fp = fix_point(__ldg(&ck.desc[pair].n2));
+  md.fs2 = fp.fs;
+  md.fl2 = fp.fl;
   md.SA = __int_as_float(h.z);
   md.C = __int_as_float(h.w);
   md.SB = __ldcg(&pm->SB);
