@@ -6,7 +6,7 @@ every compute entry point raises if the CUDA library or a B200 is missing.
 """
 from .api import ICET, Context, IcetError, Keyframe, MultiContext, Params, Result, lib_path, load_library  # noqa: F401
 from .build import build  # noqa: F401
-from .nodes import MapMakerNode, Node, OdometryNode, PointMap, ScanMatcherNode  # noqa: F401
+from .nodes import KeyframeOdometryNode, MapMakerNode, Node, OdometryNode, PointMap, ScanMatcherNode  # noqa: F401
 
 __all__ = ["ICET", "Context", "Keyframe", "MultiContext", "IcetError", "Params", "Result", "build", "load_library", "lib_path",
-           "OdometryNode", "MapMakerNode", "ScanMatcherNode", "Node", "PointMap"]
+           "OdometryNode", "MapMakerNode", "ScanMatcherNode", "Node", "PointMap", "KeyframeOdometryNode"]

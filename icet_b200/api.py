@@ -68,6 +68,36 @@ POSE_DTYPE = np.dtype([("X_homo", np.float32, (4, 4)), ("position", np.float32, 
 assert POSE_DTYPE.itemsize == C.sizeof(Pose) == 180
 
 
+class KeyframePolicy(C.Structure):
+    """icet_b200_keyframe_policy: when a scan of the keyframe odometry node becomes the next keyframe.  A scan is
+    promoted when ||X_rel[:3]|| > max_trans, max |X_rel[3:]| > max_rot, n_used < min_overlap * n_gauss1 of the keyframe,
+    max_interval scans have been registered against the keyframe, or its registration has status != 0.  A threshold
+    <= 0 turns its test off.  The defaults are those DESIGN.md §13 chose from the drift measurement."""
+    _fields_ = [("max_trans", C.c_float), ("max_rot", C.c_float), ("min_overlap", C.c_float),
+                ("max_interval", C.c_int32), ("reserved", C.c_int32 * 4)]
+
+    def __init__(self, max_trans=1.0, max_rot=0.1, min_overlap=0.5, max_interval=10):
+        for name, v in (("max_trans", max_trans), ("max_rot", max_rot), ("min_overlap", min_overlap)):
+            if not np.isfinite(v):
+                raise ValueError("policy.%s must be finite" % name)
+        if int(max_interval) != max_interval:
+            raise ValueError("policy.max_interval must be an integer")
+        super().__init__(float(max_trans), float(max_rot), float(min_overlap), int(max_interval))
+
+
+KF_TRANS, KF_ROT, KF_OVERLAP, KF_INTERVAL, KF_STATUS = 1, 2, 4, 8, 16  # icet_b200_kf_info.reason bits
+
+
+class KfInfo(C.Structure):
+    _fields_ = [("keyframe", C.c_int32), ("promoted", C.c_int32), ("reason", C.c_int32), ("x0", C.c_float * 6),
+                ("reserved", C.c_int32)]
+
+
+KF_INFO_DTYPE = np.dtype([("keyframe", np.int32), ("promoted", np.int32), ("reason", np.int32), ("x0", np.float32, 6),
+                          ("reserved", np.int32)])
+assert KF_INFO_DTYPE.itemsize == C.sizeof(KfInfo) == 40
+
+
 F32, F64, I32 = 0, 1, 2
 
 
@@ -122,7 +152,9 @@ EXPORTS = ["icet_b200_version", "icet_b200_last_error", "icet_b200_create", "ice
            "icet_b200_register_batch_multi", "icet_b200_register_sequence_multi_device", "icet_b200_multi_gathered",
            "icet_b200_multi_gathered_host", "icet_b200_keyframe_create", "icet_b200_keyframe_create_device",
            "icet_b200_keyframe_destroy", "icet_b200_keyframe_gaussians", "icet_b200_register_keyframe",
-           "icet_b200_register_keyframe_batch_device"]
+           "icet_b200_register_keyframe_batch_device", "icet_b200_kfnode_create", "icet_b200_kfnode_destroy",
+           "icet_b200_kfnode_push_device", "icet_b200_kfnode_push", "icet_b200_kfnode_push_cloud",
+           "icet_b200_kfnode_keyframe"]
 NKERNELS = 11
 
 _LIB = None
@@ -205,6 +237,15 @@ def load_library() -> C.CDLL:
     L.icet_b200_keyframe_gaussians.argtypes = [vp]
     L.icet_b200_register_keyframe.argtypes = [vp, C.POINTER(Params), vp, C.c_int32, C.c_int32, vp, C.POINTER(Result)]
     L.icet_b200_register_keyframe_batch_device.argtypes = [vp, C.POINTER(Params), C.c_int32, vp, vp, vp, vp]
+    L.icet_b200_kfnode_create.argtypes = [vp, C.POINTER(Params), C.POINTER(OdometryParams), C.POINTER(KeyframePolicy),
+                                          C.c_int32, vp, vp, C.POINTER(vp)]
+    L.icet_b200_kfnode_destroy.argtypes = [vp]
+    L.icet_b200_kfnode_push_device.argtypes = [vp, C.c_int32, vp, C.c_int32, vp, vp, vp]
+    L.icet_b200_kfnode_push.argtypes = [vp, vp, C.c_int32, C.c_int32, C.POINTER(Result), C.POINTER(Pose),
+                                        C.POINTER(KfInfo)]
+    L.icet_b200_kfnode_push_cloud.argtypes = [vp, C.POINTER(Cloud), C.POINTER(Result), C.POINTER(Pose),
+                                              C.POINTER(KfInfo)]
+    L.icet_b200_kfnode_keyframe.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_int32)]
     _LIB = L
     return L
 

@@ -12,7 +12,8 @@ LIBDIR = os.path.join(_HERE, "lib")
 LIB = os.path.join(LIBDIR, "libicet_b200.so")
 SOURCES = [os.path.join(CSRC, "icet_b200.cu")]
 DEPS = SOURCES + [os.path.join(CSRC, f) for f in ("icet_math.cuh", "synth.h", "chunk.cuh", "kernels_scan1.cuh", "kernels_pass.cuh", "kernels_pass2.cuh", "kernels_loop.cuh", "kernels_cluster.cuh",
-                                                 "runtime.inl", "callers.cuh", "callers_abi.inl", "multi_abi.inl")] + [
+                                                 "runtime.inl", "callers.cuh", "callers_abi.inl", "kernels_kfnode.cuh",
+                                                 "kfnode_abi.inl", "multi_abi.inl")] + [
     os.path.join(os.path.dirname(_HERE), "include", "icet_b200.h")]
 
 NVCC_FLAGS = [

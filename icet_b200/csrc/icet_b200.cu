@@ -42,6 +42,7 @@ namespace {
 #include "kernels_cluster.cuh"
 #include "runtime.inl"
 #include "callers.cuh"
+#include "kernels_kfnode.cuh"
 
 }  // namespace
 
@@ -842,6 +843,7 @@ int icet_b200_synth_scans_device(icet_b200_ctx* c, uint64_t seed, int32_t first_
 }
 
 #include "callers_abi.inl"
+#include "kfnode_abi.inl"
 #include "multi_abi.inl"
 
 }  // extern "C"

@@ -471,13 +471,18 @@ __global__ void __launch_bounds__(128) k_fit1(const Chunk ck) {
 // the scan-2 frames of the active voxels at R(X0) with the pair's fixed-point scale as k_fit1 does, and starts the pair like
 // k_cell_scan.  After it the scan-2 kernels see the same state as after k_fit1.  Grid: (ceil(ncell / 128), P).
 // ----------------------------------------------------------------------------------------------
+// NG: int (the keyframe's Gaussian count, known on the host) or const int32_t* (a device word: the keyframe odometry node
+// replaces its keyframe on the device, kernels_kfnode.cuh).
 static_assert(sizeof(CellRec) == 32 && sizeof(Vox1) % 8 == 0, "k_kf_attach copies CellRec as 2 float4, Vox1 as 8-byte words");
+__device__ __forceinline__ int kf_gaussians(int n) { return n; }
+__device__ __forceinline__ int kf_gaussians(const int32_t* n) { return *n; }
+template <class NG>
 __global__ void __launch_bounds__(128) k_kf_attach(const Chunk ck, const CellRec* __restrict__ krec,
-                                                   const Vox1* __restrict__ kvox, int n_gauss1) {
+                                                   const Vox1* __restrict__ kvox, NG n_gauss1) {
   pdl_prologue();
   __shared__ float s_tr[12];
   const int pair = blockIdx.y;
-  pair_start(ck, pair, n_gauss1, s_tr, blockIdx.x == 0);
+  pair_start(ck, pair, kf_gaussians(n_gauss1), s_tr, blockIdx.x == 0);
   const int c0 = blockIdx.x * 128, nc = min(128, ck.ncell - c0);
   const size_t pc = (size_t)pair * ck.ncell + c0;
   {  // flat copies of the block's cells, consecutive threads on consecutive words

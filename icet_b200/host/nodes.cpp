@@ -84,6 +84,85 @@ bool OdometryNode::pointcloudCallback(const Eigen::MatrixXf& pcl_matrix, NodeOut
   return true;
 }
 
+icet_b200_keyframe_policy KeyframeOdometryNode::defaultPolicy() {
+  icet_b200_keyframe_policy kp;
+  std::memset(&kp, 0, sizeof(kp));
+  kp.max_trans = 1.f;
+  kp.max_rot = 0.1f;
+  kp.min_overlap = 0.5f;
+  kp.max_interval = 10;
+  return kp;
+}
+
+KeyframeOdometryNode::KeyframeOdometryNode(int max_points, float minD, int run_length, int numBinsPhi, int numBinsTheta,
+                                           const icet_b200_keyframe_policy* policy, int device) {
+  X_homo = Eigen::MatrixXf::Zero(4, 4);
+  for (int k = 0; k < 4; k++) X_homo(k, k) = 1.f;
+  check(icet_b200_create(device, &ctx_));
+  icet_b200_params p;
+  std::memset(&p, 0, sizeof(p));
+  p.runlen = run_length;
+  p.bins_phi = numBinsPhi;
+  p.bins_theta = numBinsTheta;
+  p.n = 25;
+  p.thresh = 0.1f;
+  p.buff = 0.1f;
+  icet_b200_odometry_params op;
+  std::memset(&op, 0, sizeof(op));
+  op.min_range = minD;
+  op.chain_x0 = 1;
+  op.rate_hz = 10.f;
+  const icet_b200_keyframe_policy kp = policy ? *policy : defaultPolicy();
+  const int rc = icet_b200_kfnode_create(ctx_, &p, &op, &kp, max_points, nullptr, nullptr, &node_);
+  if (rc < 0) {
+    const std::string msg = std::string("ICET node: ") + icet_b200_last_error();
+    icet_b200_destroy(ctx_);
+    ctx_ = nullptr;
+    throw std::runtime_error(msg);
+  }
+}
+
+KeyframeOdometryNode::~KeyframeOdometryNode() {
+  if (node_) icet_b200_kfnode_destroy(node_);
+  if (ctx_) icet_b200_destroy(ctx_);
+}
+
+bool KeyframeOdometryNode::pointcloudCallback(const Eigen::MatrixXf& pcl_matrix, NodeOutput* out, KeyframeInfo* info) {
+  frameCount++;
+  if (pcl_matrix.rows() > 0 && pcl_matrix.cols() != 3) throw std::runtime_error("ICET node: cloud must be N x 3");
+  icet_b200_result res;
+  icet_b200_pose pose;
+  icet_b200_kf_info ki;
+  const int n = (int)pcl_matrix.rows();
+  const int rc = icet_b200_kfnode_push(node_, pcl_matrix.data(), n, n, &res, &pose, &ki);
+  check(rc);
+  if (rc == 0) return false;
+  for (int a = 0; a < 4; a++)
+    for (int b = 0; b < 4; b++) X_homo(a, b) = pose.X_homo[4 * a + b];
+  if (info) {
+    info->keyframe = ki.keyframe;
+    info->promoted = ki.promoted != 0;
+    info->reason = ki.reason;
+    for (int k = 0; k < 6; k++) info->x0[k] = ki.x0[k];
+  }
+  if (!out) return true;
+  out->X.resize(6);
+  out->pred_stds.resize(6);
+  for (int k = 0; k < 6; k++) {
+    out->X[k] = pose.X[k];
+    out->pred_stds[k] = res.pred_stds[k];
+    out->twist[k] = pose.twist[k];
+  }
+  out->X_homo = X_homo;
+  for (int k = 0; k < 3; k++) out->position[k] = pose.position[k];
+  for (int k = 0; k < 4; k++) out->orientation[k] = pose.orientation[k];
+  for (int k = 0; k < 36; k++) out->covariance[k] = 0.0;
+  for (int k = 0; k < 6; k++) out->covariance[7 * k] = pose.covariance_diag[k];
+  out->points = pose.n_points;
+  out->guarded = false;
+  return true;
+}
+
 MapMakerNode::MapMakerNode(int max_points, int map_size, int downsampleSize, int device)
     : OdometryNode(max_points, 0.2f, 12, 24, 75, device, false, 0.3f, 0.3f), map_size_(map_size),
       downsampleSize_(downsampleSize) {

@@ -146,6 +146,145 @@ class OdometryNode:
                 "twist": pose["twist"].copy(), "X_homo": pose["X_homo"].copy(), "n_points": int(pose["n_points"])}
 
 
+class KeyframeOdometryNode:
+    """Keyframe odometry (include/icet_b200.h "keyframe odometry", DESIGN.md §13): every filtered scan is registered
+    against the node's current keyframe instead of its predecessor, so the registration errors of the scans between
+    two keyframes do not add up.
+
+    * The first scan is stored unfiltered and is keyframe 0 with pose X_homo0.
+    * Scan k is filtered (||p|| > min_range) and registered against keyframe f, seeded with x0_k; its X is X_rel,
+      scan k relative to f.  Pose: X_homo_k = X_homo_f @ Hi(X_rel) (the float product of OdometryNode).
+    * Frame step: X_rel verbatim when f = k-1, else params(Hi(X_rel,k-1)^-1 Hi(X_rel,k)); twist = rate_hz * step.
+      params(H): translation column verbatim, angles from the inverse of R() (double precision).
+    * Next seed (chain_x0): params(Hi(X_rel,k) Hi(step_k)), or step_k when scan k was promoted; else 0.
+    * Scan k becomes the keyframe of scan k+1 when a test of `policy` (api.KeyframePolicy) fires or its registration
+      has status != 0.  KeyframePolicy(max_interval=1, max_trans=0, max_rot=0, min_overlap=0) reproduces
+      OdometryNode bit for bit.
+
+    `callback(scan)` returns None for the first scan, else (result, pose, info) as dicts of numpy values, info being
+    {keyframe, promoted, reason (api.KF_* bits), x0 (the seed used)}.  Nothing returns to the host between the scans of
+    one `push_device` call."""
+
+    def __init__(self, ctx: Context | None = None, max_points: int = 131072, min_range: float = 2.0, runlen: int = 7,
+                 num_bins_phi: int = 24, num_bins_theta: int = 75, rate_hz: float = 10.0, chain_x0: bool = True,
+                 policy: api.KeyframePolicy | None = None, X_homo0=None, X0=None, flags: int = 0):
+        policy = api.KeyframePolicy() if policy is None else policy
+        if not isinstance(policy, api.KeyframePolicy):
+            raise TypeError("policy must be an icet_b200.api.KeyframePolicy")
+        if any(policy.reserved):
+            raise ValueError("policy.reserved must be 0")
+        if flags & api.FLAG_CHAIN_X0:
+            raise ValueError("flags: FLAG_CHAIN_X0 is not supported by the keyframe odometry node (it seeds every "
+                             "registration itself; use chain_x0)")
+        if flags & api.FLAG_SHIPPED_ORDER:
+            raise ValueError("flags: FLAG_SHIPPED_ORDER is not supported by the keyframe odometry node (its scan-1 fit "
+                             "needs a host round trip)")
+        if max_points < 1:
+            raise ValueError("max_points must be >= 1")
+        xh = None if X_homo0 is None else np.ascontiguousarray(X_homo0, np.float32).reshape(16)
+        x0 = None if X0 is None else np.ascontiguousarray(X0, np.float32).reshape(6)
+        self.ctx = ctx or api.default_context()
+        self._L = self.ctx._L
+        self.params = api.make_params(runlen, num_bins_phi, num_bins_theta, flags=flags)
+        self.op = OdometryParams(min_range, 1 if chain_x0 else 0, rate_hz, 0.0, 0.0)
+        self.policy = policy
+        self.max_points = max_points
+        h = C.c_void_p()
+        self._h = None
+        self.ctx._check(self._L.icet_b200_kfnode_create(self.ctx._h, C.byref(self.params), C.byref(self.op),
+                                                        C.byref(policy), max_points,
+                                                        None if xh is None else xh.ctypes.data,
+                                                        None if x0 is None else x0.ctypes.data, C.byref(h)))
+        self._h = h
+        self.X_homo = np.eye(4, dtype=np.float32) if xh is None else xh.reshape(4, 4).copy()
+        self.frameCount = 0
+
+    def _handle(self):
+        if self._h is None:
+            raise IcetError("node is closed")
+        return self._h
+
+    def close(self):
+        if self._h is not None:
+            self._L.icet_b200_kfnode_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def _unpack(res, pose, info):
+        r = np.frombuffer(bytes(res), dtype=RESULT_DTYPE)[0]
+        p = np.frombuffer(bytes(pose), dtype=POSE_DTYPE)[0]
+        i = np.frombuffer(bytes(info), dtype=api.KF_INFO_DTYPE)[0]
+        return ({k: r[k].copy() for k in RESULT_DTYPE.names}, {k: p[k].copy() for k in POSE_DTYPE.names},
+                {k: i[k].copy() for k in api.KF_INFO_DTYPE.names})
+
+    def callback(self, scan):
+        """One scan from host memory (N x 3 or [3, N]), blocking."""
+        h = self._handle()
+        s = as_planes(scan)
+        res, pose, info = Result(), Pose(), api.KfInfo()
+        n = s.shape[1]
+        self.frameCount += 1
+        rc = self.ctx._check(self._L.icet_b200_kfnode_push(h, s.ctypes.data, n, n, C.byref(res), C.byref(pose),
+                                                           C.byref(info)))
+        if rc == 0:
+            return None
+        out = self._unpack(res, pose, info)
+        self.X_homo = out[1]["X_homo"].copy()
+        return out
+
+    def callback_cloud(self, cloud, divide: float = 0.0):
+        """`callback` for a cloud in its native layout (see api.cloud_desc)."""
+        h = self._handle()
+        c, keep = cloud if isinstance(cloud, tuple) else api.cloud_desc(cloud, divide)
+        res, pose, info = Result(), Pose(), api.KfInfo()
+        self.frameCount += 1
+        rc = self.ctx._check(self._L.icet_b200_kfnode_push_cloud(h, C.byref(c), C.byref(res), C.byref(pose),
+                                                                 C.byref(info)))
+        if rc == 0:
+            return None
+        out = self._unpack(res, pose, info)
+        self.X_homo = out[1]["X_homo"].copy()
+        return out
+
+    def push_device(self, scans_ptr: int, nscans: int, n: int, res_ptr: int, pose_ptr: int, info_ptr: int = 0) -> int:
+        """nscans consecutive scans in device memory [nscans, 3, n]; results (RESULT_DTYPE), poses (POSE_DTYPE) and
+        infos (KF_INFO_DTYPE, optional) to device arrays.  Asynchronous.  Returns the number of registrations."""
+        h = self._handle()
+        if nscans < 0 or n < 0 or n > self.max_points:
+            raise ValueError("nscans / n out of range")
+        return self.ctx._check(self._L.icet_b200_kfnode_push_device(h, nscans, C.c_void_p(scans_ptr), n,
+                                                                    C.c_void_p(res_ptr), C.c_void_p(pose_ptr),
+                                                                    C.c_void_p(info_ptr) if info_ptr else None))
+
+    def keyframe_device(self):
+        """(device pointer of the keyframe's filtered cloud planes, device pointer of its row count, leading dim)."""
+        p, q, ld = C.c_void_p(), C.c_void_p(), C.c_int32()
+        self.ctx._check(self._L.icet_b200_kfnode_keyframe(self._handle(), C.byref(p), C.byref(q), C.byref(ld)))
+        return p.value, q.value, ld.value
+
+    def keyframe_cloud(self) -> np.ndarray:
+        """The current keyframe's filtered cloud as an [n, 3] host array (blocking; for visualisation)."""
+        import torch
+        p, q, ld = self.keyframe_device()
+        self.ctx.synchronize()
+        n = int(torch.as_tensor(_DeviceArray(q, (1,), "<i4"), device="cuda").cpu()[0])
+        planes = torch.as_tensor(_DeviceArray(p, (3, ld), "<f4"), device="cuda")[:, :n].cpu().numpy()
+        return np.ascontiguousarray(planes.T)
+
+
+class _DeviceArray:
+    """A library-owned device buffer seen through __cuda_array_interface__ (a view, no copy; only read here)."""
+
+    def __init__(self, ptr: int, shape, typestr: str):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (ptr, False), "version": 2}
+
+
 class MapMakerNode:
     """Mirror of MapMakerNode (src/simpleMapMaker.cpp:60-291): min range 0.2 (:100), run_length 12 (:115), X0 = 0 for
     every pair (:124), divergence guard 0.3 / 0.3 (:128-137, :241-242), 2000-point random sample of every scan

@@ -363,6 +363,72 @@ int icet_b200_register_clouds(icet_b200_ctx* ctx, const icet_b200_params* p, con
 int icet_b200_node_push_cloud(icet_b200_node* node, const icet_b200_cloud* cloud, icet_b200_result* res,
                               icet_b200_pose* pose);
 
+/* -- keyframe odometry (DESIGN.md §13) --------------------------------------------------------------------------------
+ * An odometry node that registers every filtered scan against its current KEYFRAME instead of its predecessor, so
+ * that the registration errors of the scans between two keyframes do not add up.  Per scan k (after the first):
+ *   - min-range filter as in icet_b200_node_push_device; the very first scan is stored unfiltered and is keyframe 0,
+ *     with pose X_homo0;
+ *   - registration against keyframe f seeded with x0_k; its X is X_rel, scan k relative to keyframe f;
+ *   - pose X_homo_k = X_homo_f * Hi(X_rel), Hi = [R(X3,X4,X5) t; 0 1], the float product of icet_b200_node_push_device
+ *     (quaternion, covariance diagonal = pred_stds as there; twist = rate_hz * step_k; pose.X = X_rel);
+ *   - frame step step_k = X_rel verbatim when f = k-1, else params(Hi(X_rel,k-1)^-1 Hi(X_rel,k)) (both share f);
+ *     params(H) = translation column verbatim, angles from the inverse of R(), evaluated in double;
+ *   - next seed with chain_x0 = 1: params(Hi(X_rel,k) Hi(step_k)) (constant velocity), or step_k when scan k was
+ *     promoted; with chain_x0 = 0 always 0;
+ *   - promotion: scan k becomes the keyframe of scan k+1 when any enabled test of the policy fires (below) or
+ *     result.status != ICET_B200_OK.
+ * A policy that promotes every scan (max_interval = 1, other tests off) reproduces icet_b200_node_push_device bit for
+ * bit.  Filtered clouds, their sizes, the keyframe's scan-1 fit, seeds and poses stay on the device. */
+typedef struct {
+  float max_trans;      /* promote when ||X_rel[0..2]|| > max_trans (m)                                    */
+  float max_rot;        /* promote when max |X_rel[3..5]| > max_rot (rad)                                  */
+  float min_overlap;    /* promote when result.n_used < min_overlap * n_gauss1 of the keyframe             */
+  int32_t max_interval; /* promote when max_interval scans have been registered against the keyframe       */
+  int32_t reserved[4];  /* must be 0;  a threshold <= 0 turns its test off                                 */
+} icet_b200_keyframe_policy;
+
+enum { /* icet_b200_kf_info.reason: one bit per test that fired */
+  ICET_B200_KF_TRANS = 1,
+  ICET_B200_KF_ROT = 2,
+  ICET_B200_KF_OVERLAP = 4,
+  ICET_B200_KF_INTERVAL = 8,
+  ICET_B200_KF_STATUS = 16
+};
+
+typedef struct {
+  int32_t keyframe;  /* frame index of the keyframe the scan was registered against (0 = the first scan) */
+  int32_t promoted;  /* 1: this scan is the keyframe of the next one                                    */
+  int32_t reason;    /* ICET_B200_KF_* bits                                                             */
+  float x0[6];       /* the seed the registration started from                                          */
+  int32_t reserved;
+} icet_b200_kf_info; /* 10 x 4 bytes */
+
+typedef struct icet_b200_kfnode icet_b200_kfnode;
+
+/* op: min_range, chain_x0 and rate_hz as for icet_b200_node_create; guard_trans / guard_rot must be <= 0.  p must not
+ * carry ICET_B200_FLAG_CHAIN_X0 (the node seeds every registration itself) or ICET_B200_FLAG_SHIPPED_ORDER (its scan-1
+ * fit needs a host round trip).  max_points: capacity per scan (the huge-cell path of the scan-1 fit stays off below
+ * 262 144).  X_homo0 (16 floats) / x0 (6 floats, the seed of the first registration with chain_x0): HOST or NULL. */
+int icet_b200_kfnode_create(icet_b200_ctx* ctx, const icet_b200_params* p, const icet_b200_odometry_params* op,
+                            const icet_b200_keyframe_policy* kp, int32_t max_points, const float* X_homo0,
+                            const float* x0, icet_b200_kfnode** node);
+int icet_b200_kfnode_destroy(icet_b200_kfnode* node);
+/* `nscans` consecutive scans in DEVICE memory ([nscans][3][n] planes), asynchronous on the context's stream.
+ * res / poses / info: DEVICE arrays with room for nscans entries (info may be NULL).  Returns the number of
+ * registrations enqueued (nscans, or nscans - 1 on the node's first call).  Equals nscans blocking pushes byte for
+ * byte: a promotion takes effect for the very next scan. */
+int icet_b200_kfnode_push_device(icet_b200_kfnode* node, int32_t nscans, const float* scans, int32_t n,
+                                 icet_b200_result* res, icet_b200_pose* poses, icet_b200_kf_info* info);
+/* One scan in HOST memory (planes, leading dimension ld), blocking.  Returns 0 for the first scan, else 1. */
+int icet_b200_kfnode_push(icet_b200_kfnode* node, const float* scan, int32_t n, int32_t ld, icet_b200_result* res,
+                          icet_b200_pose* pose, icet_b200_kf_info* info);
+/* icet_b200_kfnode_push for a cloud in its native layout (blocking). */
+int icet_b200_kfnode_push_cloud(icet_b200_kfnode* node, const icet_b200_cloud* cloud, icet_b200_result* res,
+                                icet_b200_pose* pose, icet_b200_kf_info* info);
+/* The current keyframe's filtered cloud: device planes, leading dimension *ld, row count in device memory at *n_dev.
+ * Valid until the next push. */
+int icet_b200_kfnode_keyframe(icet_b200_kfnode* node, const float** scan, const int32_t** n_dev, int32_t* ld);
+
 /* -- multi-GPU (SURVEY.md 8e) ---------------------------------------------------------------------------------------
  * The reference's registrations are independent objects ("run multiple ICETs at once", include/icet.h:43), so a batch
  * shards by scan pair: ONE process, one context per device, device d of G registers the contiguous pair range

@@ -70,6 +70,36 @@ class ScanMatcherNode : public OdometryNode {
   Eigen::MatrixXf snailTrail;            // (:25-26, :76-80) grows by one row per registration
 };
 
+// Keyframe odometry (include/icet_b200.h "keyframe odometry", DESIGN.md §13): every filtered scan is registered against
+// the node's current keyframe; the device decides after each registration whether the scan becomes the next keyframe.
+struct KeyframeInfo {
+  int keyframe;   // frame index of the keyframe the scan was registered against
+  bool promoted;  // the scan is the keyframe of the next one
+  int reason;     // ICET_B200_KF_* bits
+  float x0[6];    // the seed the registration started from
+};
+
+class KeyframeOdometryNode {
+ public:
+  // the odometry node's constants (minD = 2, run_length = 7, 24 x 75 bins, 10 Hz twist, chained seeds) and a policy
+  // (NULL: defaultPolicy())
+  explicit KeyframeOdometryNode(int max_points = 262144, float minD = 2.f, int run_length = 7, int numBinsPhi = 24,
+                                int numBinsTheta = 75, const icet_b200_keyframe_policy* policy = nullptr, int device = 0);
+  ~KeyframeOdometryNode();
+  KeyframeOdometryNode(const KeyframeOdometryNode&) = delete;
+  KeyframeOdometryNode& operator=(const KeyframeOdometryNode&) = delete;
+  // returns false for the very first cloud (it becomes keyframe 0); out->X is X relative to the keyframe
+  bool pointcloudCallback(const Eigen::MatrixXf& pcl_matrix, NodeOutput* out, KeyframeInfo* info = nullptr);
+  static icet_b200_keyframe_policy defaultPolicy();  // 1 m, 0.1 rad, overlap 0.5, 10 scans (DESIGN.md §13)
+
+  Eigen::MatrixXf X_homo;  // host copy of the pose of the last scan
+  int frameCount = 0;
+
+ private:
+  icet_b200_ctx* ctx_ = nullptr;
+  icet_b200_kfnode* node_ = nullptr;
+};
+
 class MapMakerNode : public OdometryNode {
  public:
   // minD = 0.2 (:100), run_length = 12 (:115), X0 = 0 every time (:124), thresholds 0.3 / 0.3 (:241-242),
