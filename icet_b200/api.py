@@ -154,7 +154,8 @@ EXPORTS = ["icet_b200_version", "icet_b200_last_error", "icet_b200_create", "ice
            "icet_b200_keyframe_destroy", "icet_b200_keyframe_gaussians", "icet_b200_register_keyframe",
            "icet_b200_register_keyframe_batch_device", "icet_b200_kfnode_create", "icet_b200_kfnode_destroy",
            "icet_b200_kfnode_push_device", "icet_b200_kfnode_push", "icet_b200_kfnode_push_cloud",
-           "icet_b200_kfnode_keyframe"]
+           "icet_b200_kfnode_keyframe", "icet_b200_kfnode_create_local_map", "icet_b200_kfnode_local_map",
+           "icet_b200_kfnode_local_map_host"]
 NKERNELS = 11
 
 _LIB = None
@@ -246,6 +247,11 @@ def load_library() -> C.CDLL:
     L.icet_b200_kfnode_push_cloud.argtypes = [vp, C.POINTER(Cloud), C.POINTER(Result), C.POINTER(Pose),
                                               C.POINTER(KfInfo)]
     L.icet_b200_kfnode_keyframe.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_int32)]
+    L.icet_b200_kfnode_create_local_map.argtypes = [vp, C.POINTER(Params), C.POINTER(OdometryParams),
+                                                    C.POINTER(KeyframePolicy), C.c_int32, C.c_int32, vp, vp,
+                                                    C.POINTER(vp)]
+    L.icet_b200_kfnode_local_map.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(C.c_int32)]
+    L.icet_b200_kfnode_local_map_host.argtypes = [vp, vp, C.c_int32, C.POINTER(C.c_int32)]
     _LIB = L
     return L
 

@@ -380,6 +380,18 @@ __global__ void __launch_bounds__(256) k_ingest(const IngestDesc d, float* out, 
 // ----------------------------------------------------------------------------------------------
 // Whole-cloud re-expressions of the nodes (scanMatcher.cpp:73,76; simpleMapMaker.cpp:41,222), X read on the device.
 // ----------------------------------------------------------------------------------------------
+// One row of a re-expression: m = rot_mat.inverse() (row-major), t = trans; mode 0 `row * m - t`, mode 1 `(row - t) * m`,
+// every product and sum rounded separately (no contraction), as Eigen's float expressions are evaluated.
+__device__ __forceinline__ void xform_row(float& x, float& y, float& z, const float* m, float tx, float ty, float tz,
+                                          int mode) {
+  if (mode == 1) { x = __fsub_rn(x, tx); y = __fsub_rn(y, ty); z = __fsub_rn(z, tz); }
+  float ox = __fadd_rn(__fadd_rn(__fmul_rn(x, m[0]), __fmul_rn(y, m[3])), __fmul_rn(z, m[6]));
+  float oy = __fadd_rn(__fadd_rn(__fmul_rn(x, m[1]), __fmul_rn(y, m[4])), __fmul_rn(z, m[7]));
+  float oz = __fadd_rn(__fadd_rn(__fmul_rn(x, m[2]), __fmul_rn(y, m[5])), __fmul_rn(z, m[8]));
+  if (mode == 0) { ox = __fsub_rn(ox, tx); oy = __fsub_rn(oy, ty); oz = __fsub_rn(oz, tz); }
+  x = ox; y = oy; z = oz;
+}
+
 __global__ void __launch_bounds__(256) k_transform_cloud(const float* src, int n, int ld, const int32_t* n_dev,
                                                          const float* X, int mode, float* dst, int ld_out) {
   __shared__ float s_m[12];
@@ -393,12 +405,8 @@ __global__ void __launch_bounds__(256) k_transform_cloud(const float* src, int n
   const int rows = n_dev ? min(n, *n_dev) : n;
   const float tx = s_m[9], ty = s_m[10], tz = s_m[11];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < rows; i += gridDim.x * blockDim.x) {
-    float x = src[i], y = src[ld + i], z = src[2 * (size_t)ld + i];
-    if (mode == 1) { x = __fsub_rn(x, tx); y = __fsub_rn(y, ty); z = __fsub_rn(z, tz); }
-    float ox = __fadd_rn(__fadd_rn(__fmul_rn(x, s_m[0]), __fmul_rn(y, s_m[3])), __fmul_rn(z, s_m[6]));
-    float oy = __fadd_rn(__fadd_rn(__fmul_rn(x, s_m[1]), __fmul_rn(y, s_m[4])), __fmul_rn(z, s_m[7]));
-    float oz = __fadd_rn(__fadd_rn(__fmul_rn(x, s_m[2]), __fmul_rn(y, s_m[5])), __fmul_rn(z, s_m[8]));
-    if (mode == 0) { ox = __fsub_rn(ox, tx); oy = __fsub_rn(oy, ty); oz = __fsub_rn(oz, tz); }
+    float ox = src[i], oy = src[ld + i], oz = src[2 * (size_t)ld + i];
+    xform_row(ox, oy, oz, s_m, tx, ty, tz, mode);
     dst[i] = ox;
     dst[ld_out + i] = oy;
     dst[2 * (size_t)ld_out + i] = oz;

@@ -7,6 +7,9 @@
 //   candidate fit    chunk_setup + chunk_scan1 on that descriptor (n1 = 0 unless scan k was promoted)
 //   k_kf_commit      promoted: the candidate's CellRec / Vox1 and n_gauss1 become the node's keyframe
 //   k_copy_cloud     promoted: the filtered cloud becomes the node's keyframe cloud (0 rows otherwise)
+// A local-map node (icet_b200_kfnode_create_local_map, DESIGN.md §14) fits the merged clouds of its last M keyframes
+// instead of the promoted scan alone: k_lmap_window and k_lmap_assemble run between k_kfnode_step and the candidate
+// fit, which then reads the map (n1max = M * cap).
 #pragma once
 
 struct KfNodeState {        // device-resident members of the keyframe odometry node
@@ -155,9 +158,10 @@ __global__ void __launch_bounds__(32) k_kfnode_step(KfNodeState* st, const icet_
 // The candidate fit becomes the keyframe (when the step kernel promoted its scan): flat 16-byte copies of its CellRec
 // and Vox1 records (one 8-byte tail word when ncell * sizeof(Vox1) is not a multiple of 16) and its Gaussian count.
 static_assert(sizeof(CellRec) % 16 == 0 && sizeof(Vox1) % 8 == 0, "k_kf_commit copies 16-byte words (+ one 8-byte tail)");
+// kf_rows: rows of the promoted keyframe's own cloud (the fit's n1 for a plain node; a local-map node fits more rows).
 __global__ void __launch_bounds__(256) k_kf_commit(KfNodeState* st, const CellRec* __restrict__ crec,
                                                    const Vox1* __restrict__ cvox, const icet_b200_result* cres,
-                                                   const PairDesc* fit, CellRec* krec, Vox1* kvox, int ncell) {
+                                                   const int32_t* kf_rows, CellRec* krec, Vox1* kvox, int ncell) {
   if (!st->commit) return;
   const int nr = ncell * (int)(sizeof(CellRec) / 16);
   const size_t vb = (size_t)ncell * sizeof(Vox1);
@@ -173,7 +177,101 @@ __global__ void __launch_bounds__(256) k_kf_commit(KfNodeState* st, const CellRe
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     if (vb % 16) reinterpret_cast<uint2*>(kvox)[vb / 8 - 1] = reinterpret_cast<const uint2*>(cvox)[vb / 8 - 1];
     st->n_gauss1 = cres->n_gauss1;
-    st->kf_n = fit->n1;
+    st->kf_n = *kf_rows;
+  }
+}
+
+// -- local map (DESIGN.md §14) ---------------------------------------------------------------------------------------
+// A ring of M keyframe slots: the original filtered cloud of each keyframe ([M][3][cap], owned by the host struct),
+// its row count and its transform into the frame of the newest keyframe.  The map lists the slots newest first.
+constexpr int LMAP_MAX = 16;
+constexpr long long LMAP_MAX_ROWS = 1LL << 28;  // map capacity M * cap: int32 row offsets and tile grids stay far from 2^31
+
+struct LmapState {
+  double T[LMAP_MAX][16];     // ring slot -> current keyframe frame, on column vectors: p_cur = T p_slot (row-major)
+  float m[LMAP_MAX][12];      // map block b: T of its slot as k_transform_cloud mode 0 takes it, `row * m[0..8] - m[9..11]`
+  int32_t n[LMAP_MAX];        // rows of each ring slot
+  int32_t src[LMAP_MAX];      // map block b -> ring slot
+  int32_t off[LMAP_MAX + 1];  // map block b -> its first map row; off[count] = map_n
+  int32_t head;               // ring slot of the newest keyframe
+  int32_t count;              // keyframes in the window (<= M)
+  int32_t nblk;               // blocks k_lmap_assemble writes for the scan just stepped (0: it was not promoted)
+  int32_t newest_n;           // rows of the keyframe promoted by that scan (0: none)
+  int32_t map_n;              // rows of the map
+};
+
+// After k_kfnode_step: when it promoted scan k, re-express the window in k's frame and give k the next ring slot.
+// The registration of k against keyframe f maps a point p of k into f as (p + t) R(X) (row vectors), so a point q of
+// f is q R^-1 - t in k's frame (k_transform_cloud mode 0): F = [R t'; 0 1] with t' = -t on column vectors (R^-T = R
+// for a rotation), and every slot's T becomes F T, composed in double.  Lane j composes the j-th newest slot.
+__global__ void __launch_bounds__(32) k_lmap_window(const KfNodeState* st, LmapState* lm, const icet_b200_result* res,
+                                                    const int32_t* kept, int M) {
+  const int lane = threadIdx.x;
+  if (!st->commit) {
+    if (lane == 0) { lm->nblk = 0; lm->newest_n = 0; }
+    return;
+  }
+  const int head = lm->head, count = lm->count;
+  if (res && lane < count) {
+    double F[16], T[16];
+    kf_homo(res->X, F);
+    F[3] = -F[3]; F[7] = -F[7]; F[11] = -F[11];
+    double* Ts = lm->T[(head - lane + M) % M];
+    kf_mul(F, Ts, T);
+    for (int k = 0; k < 16; k++) Ts[k] = T[k];
+  }
+  __syncwarp();
+  if (lane != 0) return;
+  const int h = (head + 1) % M, cnt = min(count + 1, M);  // a full ring retires its oldest slot, h
+  for (int k = 0; k < 16; k++) lm->T[h][k] = (k % 5 == 0) ? 1.0 : 0.0;
+  lm->n[h] = *kept;
+  int off = 0;
+  for (int b = 0; b < cnt; b++) {
+    const int s = (h - b + M) % M;
+    const double* T = lm->T[s];
+    for (int r = 0; r < 3; r++)
+      for (int c = 0; c < 3; c++) lm->m[b][3 * r + c] = (float)T[4 * c + r];
+    lm->m[b][9] = (float)-T[3]; lm->m[b][10] = (float)-T[7]; lm->m[b][11] = (float)-T[11];
+    lm->src[b] = s;
+    lm->off[b] = off;
+    off += lm->n[s];
+  }
+  lm->off[cnt] = off;
+  lm->head = h; lm->count = cnt; lm->nblk = cnt; lm->newest_n = *kept; lm->map_n = off;
+}
+
+// The map, one block row per window slot (blockIdx.y = b, newest first, no gaps): block 0 is the promoted scan's
+// filtered cloud, copied verbatim into the map and into its ring slot; the others are their slot's stored cloud through
+// the mode-0 arithmetic of k_transform_cloud.  Writes the candidate-fit descriptor (scan 1 = the map).  Nothing when
+// the scan was not promoted: k_kfnode_step's descriptor (n1 = 0) stands.
+__global__ void __launch_bounds__(256) k_lmap_assemble(const LmapState* lm, const float* slot, int cap, float* ring,
+                                                       float* map, int ldm, PairDesc* fit) {
+  const int b = blockIdx.y;
+  if (b >= lm->nblk) return;
+  const int s = lm->src[b], n = lm->n[s], o = lm->off[b];
+  float m[12];
+  for (int k = 0; k < 12; k++) m[k] = lm->m[b][k];
+  const float* src = b == 0 ? slot : ring + (size_t)s * 3 * cap;
+  float* keep = ring + (size_t)s * 3 * cap;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    float x = src[i], y = src[cap + i], z = src[2 * (size_t)cap + i];
+    if (b == 0) {
+      keep[i] = x; keep[cap + i] = y; keep[2 * (size_t)cap + i] = z;
+    } else {
+      xform_row(x, y, z, m, m[9], m[10], m[11], 0);
+    }
+    map[o + i] = x; map[ldm + o + i] = y; map[2 * (size_t)ldm + o + i] = z;
+  }
+  if (b == 0 && blockIdx.x == 0 && threadIdx.x == 0) {
+    PairDesc d;
+    d.s1 = map; d.n1 = lm->map_n; d.ld1 = ldm; d.s2 = nullptr; d.n2 = 0; d.ld2 = 0;
+    *fit = d;
+  }
+}
+
+__global__ void k_lmap_init(LmapState* lm, int M) {
+  if (threadIdx.x == 0) {
+    lm->head = M - 1; lm->count = 0; lm->nblk = 0; lm->newest_n = 0; lm->map_n = 0;
   }
 }
 

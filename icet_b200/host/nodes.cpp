@@ -95,7 +95,7 @@ icet_b200_keyframe_policy KeyframeOdometryNode::defaultPolicy() {
 }
 
 KeyframeOdometryNode::KeyframeOdometryNode(int max_points, float minD, int run_length, int numBinsPhi, int numBinsTheta,
-                                           const icet_b200_keyframe_policy* policy, int device) {
+                                           const icet_b200_keyframe_policy* policy, int device, int map_keyframes) {
   X_homo = Eigen::MatrixXf::Zero(4, 4);
   for (int k = 0; k < 4; k++) X_homo(k, k) = 1.f;
   check(icet_b200_create(device, &ctx_));
@@ -113,7 +113,10 @@ KeyframeOdometryNode::KeyframeOdometryNode(int max_points, float minD, int run_l
   op.chain_x0 = 1;
   op.rate_hz = 10.f;
   const icet_b200_keyframe_policy kp = policy ? *policy : defaultPolicy();
-  const int rc = icet_b200_kfnode_create(ctx_, &p, &op, &kp, max_points, nullptr, nullptr, &node_);
+  const int rc = map_keyframes == 0
+                     ? icet_b200_kfnode_create(ctx_, &p, &op, &kp, max_points, nullptr, nullptr, &node_)
+                     : icet_b200_kfnode_create_local_map(ctx_, &p, &op, &kp, map_keyframes, max_points, nullptr,
+                                                         nullptr, &node_);
   if (rc < 0) {
     const std::string msg = std::string("ICET node: ") + icet_b200_last_error();
     icet_b200_destroy(ctx_);
@@ -125,6 +128,14 @@ KeyframeOdometryNode::KeyframeOdometryNode(int max_points, float minD, int run_l
 KeyframeOdometryNode::~KeyframeOdometryNode() {
   if (node_) icet_b200_kfnode_destroy(node_);
   if (ctx_) icet_b200_destroy(ctx_);
+}
+
+Eigen::MatrixXf KeyframeOdometryNode::localMap() {
+  int32_t n = 0;
+  check(icet_b200_kfnode_local_map_host(node_, nullptr, 0, &n));
+  Eigen::MatrixXf out(n, 3);
+  if (n > 0) check(icet_b200_kfnode_local_map_host(node_, out.data(), n, &n));
+  return out;
 }
 
 bool KeyframeOdometryNode::pointcloudCallback(const Eigen::MatrixXf& pcl_matrix, NodeOutput* out, KeyframeInfo* info) {

@@ -163,11 +163,21 @@ class KeyframeOdometryNode:
 
     `callback(scan)` returns None for the first scan, else (result, pose, info) as dicts of numpy values, info being
     {keyframe, promoted, reason (api.KF_* bits), x0 (the seed used)}.  Nothing returns to the host between the scans of
-    one `push_device` call."""
+    one `push_device` call.
+
+    Local map (DESIGN.md §14): with `map_keyframes=M` (1 <= M <= 16) scan 1 of every registration is the local map
+    instead of the keyframe alone: the filtered clouds of the last M keyframes in the frame of the newest keyframe f.
+    Its rows are f's cloud (bit for bit), then the older keyframes, newest to oldest, without gaps.  On a promotion of
+    scan k a point q of f's frame becomes q R(X_rel)^-1 - t(X_rel) in k's frame (Context.transform_cloud_device mode
+    0); each keyframe keeps its original filtered cloud and its transform into the current frame, composed in double
+    on the device, so a map is never re-expressed twice.  Pose, seeds, policy and info are those above; the overlap
+    test uses the map's n_gauss1.  The window slides once M keyframes exist.  M = 1 is the plain node byte for byte;
+    `None` (the default) creates the plain node through icet_b200_kfnode_create."""
 
     def __init__(self, ctx: Context | None = None, max_points: int = 131072, min_range: float = 2.0, runlen: int = 7,
                  num_bins_phi: int = 24, num_bins_theta: int = 75, rate_hz: float = 10.0, chain_x0: bool = True,
-                 policy: api.KeyframePolicy | None = None, X_homo0=None, X0=None, flags: int = 0):
+                 policy: api.KeyframePolicy | None = None, X_homo0=None, X0=None, flags: int = 0,
+                 map_keyframes: int | None = None):
         policy = api.KeyframePolicy() if policy is None else policy
         if not isinstance(policy, api.KeyframePolicy):
             raise TypeError("policy must be an icet_b200.api.KeyframePolicy")
@@ -181,6 +191,8 @@ class KeyframeOdometryNode:
                              "needs a host round trip)")
         if max_points < 1:
             raise ValueError("max_points must be >= 1")
+        if map_keyframes is not None and not 1 <= map_keyframes <= 16:
+            raise ValueError("map_keyframes must be in 1 .. 16")
         xh = None if X_homo0 is None else np.ascontiguousarray(X_homo0, np.float32).reshape(16)
         x0 = None if X0 is None else np.ascontiguousarray(X0, np.float32).reshape(6)
         self.ctx = ctx or api.default_context()
@@ -189,12 +201,17 @@ class KeyframeOdometryNode:
         self.op = OdometryParams(min_range, 1 if chain_x0 else 0, rate_hz, 0.0, 0.0)
         self.policy = policy
         self.max_points = max_points
+        self.map_keyframes = map_keyframes
         h = C.c_void_p()
         self._h = None
-        self.ctx._check(self._L.icet_b200_kfnode_create(self.ctx._h, C.byref(self.params), C.byref(self.op),
-                                                        C.byref(policy), max_points,
-                                                        None if xh is None else xh.ctypes.data,
-                                                        None if x0 is None else x0.ctypes.data, C.byref(h)))
+        pointers = (None if xh is None else xh.ctypes.data, None if x0 is None else x0.ctypes.data, C.byref(h))
+        if map_keyframes is None:
+            rc = self._L.icet_b200_kfnode_create(self.ctx._h, C.byref(self.params), C.byref(self.op), C.byref(policy),
+                                                 max_points, *pointers)
+        else:
+            rc = self._L.icet_b200_kfnode_create_local_map(self.ctx._h, C.byref(self.params), C.byref(self.op),
+                                                           C.byref(policy), map_keyframes, max_points, *pointers)
+        self.ctx._check(rc)
         self._h = h
         self.X_homo = np.eye(4, dtype=np.float32) if xh is None else xh.reshape(4, 4).copy()
         self.frameCount = 0
@@ -270,8 +287,21 @@ class KeyframeOdometryNode:
 
     def keyframe_cloud(self) -> np.ndarray:
         """The current keyframe's filtered cloud as an [n, 3] host array (blocking; for visualisation)."""
+        return self._host_cloud(*self.keyframe_device())
+
+    def local_map_device(self):
+        """(device pointer of the local map's planes, device pointer of its row count, leading dim): scan 1 of the next
+        registration, valid until the next push.  The keyframe cloud for a node made without map_keyframes."""
+        p, q, ld = C.c_void_p(), C.c_void_p(), C.c_int32()
+        self.ctx._check(self._L.icet_b200_kfnode_local_map(self._handle(), C.byref(p), C.byref(q), C.byref(ld)))
+        return p.value, q.value, ld.value
+
+    def local_map_cloud(self) -> np.ndarray:
+        """The local map as an [n, 3] host array (blocking)."""
+        return self._host_cloud(*self.local_map_device())
+
+    def _host_cloud(self, p, q, ld) -> np.ndarray:
         import torch
-        p, q, ld = self.keyframe_device()
         self.ctx.synchronize()
         n = int(torch.as_tensor(_DeviceArray(q, (1,), "<i4"), device="cuda").cpu()[0])
         planes = torch.as_tensor(_DeviceArray(p, (3, ld), "<f4"), device="cuda")[:, :n].cpu().numpy()

@@ -429,6 +429,32 @@ int icet_b200_kfnode_push_cloud(icet_b200_kfnode* node, const icet_b200_cloud* c
  * Valid until the next push. */
 int icet_b200_kfnode_keyframe(icet_b200_kfnode* node, const float** scan, const int32_t** n_dev, int32_t* ld);
 
+/* Local-map keyframe odometry (DESIGN.md §14): a keyframe odometry node whose scan 1 is the LOCAL MAP, the filtered
+ * clouds of its last map_keyframes = M keyframes (1 <= M <= 16) expressed in the frame of the newest keyframe f.
+ * Pose, frame step, seeds, promotion policy, icet_b200_kf_info and the rejections are those above; the overlap test
+ * uses the map's n_gauss1 (the result's).  The map:
+ *   - rows of f first, bit for bit as icet_b200_kfnode_keyframe holds them; then the older keyframes, newest to
+ *     oldest; no gaps; row count = the sum of the window's kept counts, in device memory.  (Results do not depend on
+ *     the row order; it is fixed so that maps compare byte for byte.)
+ *   - Re-expression: registering scan k against f maps p of k into f as (p + t) R(X) (row vectors), so on promotion of
+ *     k a point q of f's frame is q R^-1 - t in k's frame (icet_b200_transform_cloud_device mode 0).  Each window
+ *     keyframe keeps its original filtered cloud and its transform into the current keyframe frame, composed in double
+ *     on the device and applied in float to that original cloud (never to an already re-expressed map).  These
+ *     transforms are not derived from the published pose X_homo.
+ *   - The window slides: after the (M+1)-th keyframe the oldest leaves it; before M keyframes it holds those there are.
+ * M = 1 is icet_b200_kfnode_create byte for byte.  max_points: capacity per scan; M * max_points must not exceed 2^28
+ * (the huge-cell path of the candidate fit is on once M * max_points exceeds 262 144).  Everything else as
+ * icet_b200_kfnode_create; push / keyframe / destroy take the node as they are. */
+int icet_b200_kfnode_create_local_map(icet_b200_ctx* ctx, const icet_b200_params* p, const icet_b200_odometry_params* op,
+                                      const icet_b200_keyframe_policy* kp, int32_t map_keyframes, int32_t max_points,
+                                      const float* X_homo0, const float* x0, icet_b200_kfnode** node);
+/* The current local map (scan 1 of the next registration): device planes, leading dimension *ld, row count in device
+ * memory at *n_dev.  Valid until the next push.  For a node of icet_b200_kfnode_create: its keyframe cloud. */
+int icet_b200_kfnode_local_map(icet_b200_kfnode* node, const float** cloud, const int32_t** n_dev, int32_t* ld);
+/* The same in HOST memory, blocking: *n_out = its row count; with out != NULL the x | y | z planes (leading dimension
+ * ld_out >= *n_out) as well.  Call with out = NULL to size the buffer. */
+int icet_b200_kfnode_local_map_host(icet_b200_kfnode* node, float* out, int32_t ld_out, int32_t* n_out);
+
 /* -- multi-GPU (SURVEY.md 8e) ---------------------------------------------------------------------------------------
  * The reference's registrations are independent objects ("run multiple ICETs at once", include/icet.h:43), so a batch
  * shards by scan pair: ONE process, one context per device, device d of G registers the contiguous pair range

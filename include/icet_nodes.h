@@ -82,15 +82,18 @@ struct KeyframeInfo {
 class KeyframeOdometryNode {
  public:
   // the odometry node's constants (minD = 2, run_length = 7, 24 x 75 bins, 10 Hz twist, chained seeds) and a policy
-  // (NULL: defaultPolicy())
+  // (NULL: defaultPolicy()).  map_keyframes = M in 1 .. 16: scan 1 of every registration is the local map of the last M
+  // keyframes (icet_b200_kfnode_create_local_map, DESIGN.md §14); 0: the keyframe alone.
   explicit KeyframeOdometryNode(int max_points = 262144, float minD = 2.f, int run_length = 7, int numBinsPhi = 24,
-                                int numBinsTheta = 75, const icet_b200_keyframe_policy* policy = nullptr, int device = 0);
+                                int numBinsTheta = 75, const icet_b200_keyframe_policy* policy = nullptr, int device = 0,
+                                int map_keyframes = 0);
   ~KeyframeOdometryNode();
   KeyframeOdometryNode(const KeyframeOdometryNode&) = delete;
   KeyframeOdometryNode& operator=(const KeyframeOdometryNode&) = delete;
   // returns false for the very first cloud (it becomes keyframe 0); out->X is X relative to the keyframe
   bool pointcloudCallback(const Eigen::MatrixXf& pcl_matrix, NodeOutput* out, KeyframeInfo* info = nullptr);
   static icet_b200_keyframe_policy defaultPolicy();  // 1 m, 0.1 rad, overlap 0.5, 10 scans (DESIGN.md §13)
+  Eigen::MatrixXf localMap();  // N x 3: scan 1 of the next registration (the keyframe cloud when map_keyframes = 0)
 
   Eigen::MatrixXf X_homo;  // host copy of the pose of the last scan
   int frameCount = 0;
