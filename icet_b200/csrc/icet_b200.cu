@@ -23,6 +23,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -73,7 +74,7 @@ int icet_b200_create(int device, icet_b200_ctx** out) {
     return fail(ICET_B200_E_NODEVICE, std::string("device '") + prop.name + "' is sm_" + std::to_string(prop.major) +
                                           std::to_string(prop.minor) + "; this library is built for sm_100a only");
   CK(cudaSetDevice(device));
-  icet_b200_ctx* c = new icet_b200_ctx();
+  Building<icet_b200_ctx> c(new icet_b200_ctx(), icet_b200_destroy);
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
   if (const char* e = getenv("ICET_B200_LOOP_TIMEOUT_MS")) {
@@ -98,37 +99,30 @@ int icet_b200_create(int device, icet_b200_ctx** out) {
     CK(cudaEventCreateWithFlags(&c->ev_copy[i], cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&c->ev_done[i], cudaEventDisableTiming));
   }
-  *out = c;
+  *out = c.release();
   return 0;
 }
 
 int icet_b200_destroy(icet_b200_ctx* c) {
   if (!c) return 0;
   cudaSetDevice(c->device);
-  cudaStreamSynchronize(c->stream);
-  cudaStreamSynchronize(c->copy_stream);
+  if (c->stream) cudaStreamSynchronize(c->stream);
+  if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
   for (int l = 1; l < ICET_NLANE; l++)
     if (c->lanes[l]) cudaStreamSynchronize(c->lanes[l]);
-  for (int i = 0; i < ICET_NLANE; i++) c->ws[i].release();
-  c->edges.release(); c->resbuf.release(); c->dumpbuf.release(); c->posebuf.release();
-  c->rawbuf[0].release(); c->rawbuf[1].release(); c->planebuf.release();
   for (int i = 0; i < ICET_NSLOT; i++) {
-    c->stage[i].release(); c->descbuf[i].release(); c->x0buf[i].release();
     if (c->ev_copy[i]) cudaEventDestroy(c->ev_copy[i]);
     if (c->ev_done[i]) cudaEventDestroy(c->ev_done[i]);
   }
   for (cudaEvent_t e : c->prof_ev) cudaEventDestroy(e);
-  if (c->pinned) cudaFreeHost(c->pinned);
   if (c->own_stream && c->stream) cudaStreamDestroy(c->stream);
   if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
   for (int l = 1; l < ICET_NLANE; l++) {
     if (c->lanes[l]) cudaStreamDestroy(c->lanes[l]);
     if (c->ev_join[l]) cudaEventDestroy(c->ev_join[l]);
   }
-  for (int l = 0; l < ICET_NLANE; l++) {
-    c->lane_desc[l].release();
+  for (int l = 0; l < ICET_NLANE; l++)
     if (c->ev_lane[l]) cudaEventDestroy(c->ev_lane[l]);
-  }
   if (c->ev_fork) cudaEventDestroy(c->ev_fork);
   for (int k = 0; k < 2; k++)
     if (c->ev_aux[k]) cudaEventDestroy(c->ev_aux[k]);
@@ -225,6 +219,18 @@ int icet_b200_set_dump(icet_b200_ctx* c, int32_t enable) {
 }
 
 // -- device-resident batch --------------------------------------------------------------------
+// The pair arrays of a batch: present, and every pair with sizes >= 0 and a scan wherever it has points.  Without
+// scan 1 (with_scan1 false: a batch against a keyframe) scan1 and n1 are not read.
+static int check_pairs(int32_t npairs, bool with_scan1, const float* const* scan1, const int32_t* n1,
+                       const float* const* scan2, const int32_t* n2, const icet_b200_result* out) {
+  if (npairs < 0 || (npairs > 0 && ((with_scan1 && (!scan1 || !n1)) || !scan2 || !n2 || !out)))
+    return fail(ICET_B200_E_INVALID, "NULL argument");
+  for (int i = 0; i < npairs; i++)
+    if ((with_scan1 && (n1[i] < 0 || (n1[i] > 0 && !scan1[i]))) || n2[i] < 0 || (n2[i] > 0 && !scan2[i]))
+      return fail(ICET_B200_E_INVALID, "bad scan pointer / size in pair " + std::to_string(i));
+  return 0;
+}
+
 static int batch_device_impl(icet_b200_ctx* c, const icet_b200_params* p, int32_t npairs, const PairDesc* h_desc,
                              const float* d_x0, icet_b200_result* d_out, bool dump, const PairDesc* d_desc_all = nullptr,
                              int nmax_dev = 0, const icet_b200_keyframe* kf = nullptr) {
@@ -232,7 +238,7 @@ static int batch_device_impl(icet_b200_ctx* c, const icet_b200_params* p, int32_
   // d_desc_all (callers layer): the descriptors are already on the device -- built there, with data-dependent
   // sizes no larger than nmax_dev -- and h_desc is not read.
   // kf: scan 1 of every pair is this keyframe (the descriptors hold no scan 1).
-  int rc = ensure_pinned(c, (size_t)std::min(npairs, c->chunk_pairs) * sizeof(PairDesc) * ICET_NLANE + 4096);
+  int rc = c->pinned.ensure((size_t)std::min(npairs, c->chunk_pairs) * sizeof(PairDesc) * ICET_NLANE + 4096);
   if (rc) return rc;
   // consecutive chunks alternate between the two compute lanes (own stream + workspace each); lane 1 starts after
   // everything already queued on the caller's stream and the caller's stream resumes after lane 1
@@ -271,7 +277,7 @@ static int batch_device_impl(icet_b200_ctx* c, const icet_b200_params* p, int32_
       if (rc) return rc;
       // the pinned part of this lane may still be in flight from its previous chunk
       CK(cudaEventSynchronize(c->ev_lane[slot]));
-      PairDesc* hp = (PairDesc*)c->pinned + (size_t)slot * std::min(npairs, c->chunk_pairs);
+      PairDesc* hp = (PairDesc*)c->pinned.p + (size_t)slot * std::min(npairs, c->chunk_pairs);
       memcpy(hp, h_desc + base, (size_t)P * sizeof(PairDesc));
       CK(cudaMemcpyAsync(c->lane_desc[slot].p, hp, (size_t)P * sizeof(PairDesc), cudaMemcpyHostToDevice, st));
       CK(cudaEventRecord(c->ev_lane[slot], st));
@@ -294,17 +300,12 @@ int icet_b200_register_batch_device(icet_b200_ctx* c, const icet_b200_params* p,
                                     const int32_t* n2, const float* x0, icet_b200_result* out) {
   if (!c) return fail(ICET_B200_E_INVALID, "ctx is NULL");
   int rc = validate(p);
+  if (!rc) rc = check_pairs(npairs, true, scan1, n1, scan2, n2, out);
   if (rc) return rc;
-  if (npairs < 0 || (npairs > 0 && (!scan1 || !scan2 || !n1 || !n2 || !out)))
-    return fail(ICET_B200_E_INVALID, "NULL argument");
   if (npairs == 0) return 0;
   CK(cudaSetDevice(c->device));
   std::vector<PairDesc> d(npairs);
-  for (int i = 0; i < npairs; i++) {
-    if (n1[i] < 0 || n2[i] < 0 || (n1[i] > 0 && !scan1[i]) || (n2[i] > 0 && !scan2[i]))
-      return fail(ICET_B200_E_INVALID, "bad scan pointer / size in pair " + std::to_string(i));
-    d[i] = PairDesc{scan1[i], scan2[i], n1[i], n1[i], n2[i], n2[i]};
-  }
+  for (int i = 0; i < npairs; i++) d[i] = PairDesc{scan1[i], scan2[i], n1[i], n1[i], n2[i], n2[i]};
   return batch_device_impl(c, p, npairs, d.data(), x0, out, false);
 }
 
@@ -328,13 +329,9 @@ int icet_b200_register_batch(icet_b200_ctx* c, const icet_b200_params* p, int32_
                              const int32_t* n2, const float* x0, icet_b200_result* out) {
   if (!c) return fail(ICET_B200_E_INVALID, "ctx is NULL");
   int rc = validate(p);
+  if (!rc) rc = check_pairs(npairs, true, scan1, n1, scan2, n2, out);
   if (rc) return rc;
-  if (npairs < 0 || (npairs > 0 && (!scan1 || !scan2 || !n1 || !n2 || !out)))
-    return fail(ICET_B200_E_INVALID, "NULL argument");
   if (npairs == 0) return 0;
-  for (int i = 0; i < npairs; i++)
-    if (n1[i] < 0 || n2[i] < 0 || (n1[i] > 0 && !scan1[i]) || (n2[i] > 0 && !scan2[i]))
-      return fail(ICET_B200_E_INVALID, "bad scan pointer / size in pair " + std::to_string(i));
   CK(cudaSetDevice(c->device));
   rc = c->resbuf.ensure((size_t)npairs * sizeof(icet_b200_result));
   if (rc) return rc;
@@ -362,7 +359,7 @@ int icet_b200_register_batch(icet_b200_ctx* c, const icet_b200_params* p, int32_
     for (size_t k = tail.size(); k-- > 0;) sizes.push_back(tail[k]);
   }
   const size_t pin_slot = (size_t)CH * (sizeof(PairDesc) + 6 * sizeof(float)) + 2048;
-  rc = ensure_pinned(c, pin_slot * ICET_NSLOT + 4096);
+  rc = c->pinned.ensure(pin_slot * ICET_NSLOT + 4096);
   if (rc) return rc;
   auto pad = [](size_t f) { return (f + 63) & ~(size_t)63; };
   int base = 0;
@@ -447,7 +444,7 @@ int icet_b200_register_batch(icet_b200_ctx* c, const icet_b200_params* p, int32_
     rc = flush();
     if (rc) return rc;
     prev_scan2_dev = sbase + off2[P - 1];
-    char* hp = (char*)c->pinned + (size_t)slot * pin_slot;
+    char* hp = (char*)c->pinned.p + (size_t)slot * pin_slot;
     memcpy(hp, d.data(), (size_t)P * sizeof(PairDesc));
     CK(cudaMemcpyAsync(c->descbuf[slot].p, hp, (size_t)P * sizeof(PairDesc), cudaMemcpyHostToDevice, c->copy_stream));
     const float* d_x0 = nullptr;
@@ -478,7 +475,6 @@ int icet_b200_register_batch(icet_b200_ctx* c, const icet_b200_params* p, int32_
     }
     if (npairs == 1) {
       c->last_n2 = n2[0];
-      c->last_runlen = p->runlen;
       c->last_valid = true;
     }
   }
@@ -527,16 +523,14 @@ static int keyframe_params(const icet_b200_keyframe* kf, const icet_b200_params*
   return 0;
 }
 
-// Copies a HOST cloud (planes, leading dimension ld) into n-strided DEVICE planes at dst.
-static int upload_planes(icet_b200_ctx* c, float* dst, const float* src, int32_t n, int32_t ld) {
+// Copies a HOST cloud (planes, leading dimension ld) into n-strided DEVICE planes at dst, on the context's stream.
+static int upload_cloud(icet_b200_ctx* c, float* dst, const float* src, int32_t n, int32_t ld) {
   if (n == 0) return 0;
-  if (ld == n) {
+  if (ld == n)
     CK(cudaMemcpyAsync(dst, src, (size_t)3 * n * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    return 0;
-  }
-  for (int k = 0; k < 3; k++)
-    CK(cudaMemcpyAsync(dst + (size_t)k * n, src + (size_t)k * ld, (size_t)n * sizeof(float), cudaMemcpyHostToDevice,
-                       c->stream));
+  else
+    CK(cudaMemcpy2DAsync(dst, (size_t)n * sizeof(float), src, (size_t)ld * sizeof(float), (size_t)n * sizeof(float), 3,
+                         cudaMemcpyHostToDevice, c->stream));
   return 0;
 }
 
@@ -553,14 +547,14 @@ int icet_b200_keyframe_create_device(icet_b200_ctx* c, const icet_b200_params* p
   icet_b200_params q = *p;
   q.runlen = 0;
   q.flags = p->flags & ICET_B200_FLAG_SHIPPED_ORDER;
-  rc = ensure_pinned(c, 4096);
+  rc = c->pinned.ensure(4096);
   if (rc) return rc;
   rc = c->descbuf[0].ensure(sizeof(PairDesc));
   if (rc) return rc;
   rc = c->resbuf.ensure(sizeof(icet_b200_result));
   if (rc) return rc;
   CK(cudaStreamSynchronize(c->stream));  // the pinned bounce buffer may still feed an earlier upload
-  PairDesc* hd = (PairDesc*)c->pinned;
+  PairDesc* hd = (PairDesc*)c->pinned.p;
   *hd = PairDesc{scan1, nullptr, n1, ld1, 0, 0};
   CK(cudaMemcpyAsync(c->descbuf[0].p, hd, sizeof(PairDesc), cudaMemcpyHostToDevice, c->stream));
   icet_b200_result* d_res = (icet_b200_result*)c->resbuf.p;
@@ -570,29 +564,21 @@ int icet_b200_keyframe_create_device(icet_b200_ctx* c, const icet_b200_params* p
   c->last_valid = false;  // lane 0's workspace now holds this chunk
   if (rc) return rc;
   CK(cudaGetLastError());
-  icet_b200_keyframe* kf = new icet_b200_keyframe();
+  Building<icet_b200_keyframe> kf(new icet_b200_keyframe(), icet_b200_keyframe_destroy);
   kf->ctx = c;
   kf->p = q;
   const size_t ncell = (size_t)p->bins_phi * p->bins_theta;
-  rc = kf->rec.ensure(ncell * sizeof(CellRec));
-  if (!rc) rc = kf->vox.ensure(ncell * sizeof(Vox1));
-  if (rc) {
-    icet_b200_keyframe_destroy(kf);
-    return rc;
-  }
-  int32_t* h_ng = (int32_t*)((char*)c->pinned + 1024);
+  if ((rc = kf->rec.ensure(ncell * sizeof(CellRec))) || (rc = kf->vox.ensure(ncell * sizeof(Vox1)))) return rc;
+  int32_t* h_ng = (int32_t*)((char*)c->pinned.p + 1024);
   cudaError_t e = cudaMemcpyAsync(kf->rec.p, r.ck.rec, ncell * sizeof(CellRec), cudaMemcpyDeviceToDevice, c->stream);
   if (e == cudaSuccess)
     e = cudaMemcpyAsync(kf->vox.p, r.ck.vox, ncell * sizeof(Vox1), cudaMemcpyDeviceToDevice, c->stream);
   if (e == cudaSuccess)
     e = cudaMemcpyAsync(h_ng, &d_res->n_gauss1, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  if (e != cudaSuccess) {
-    icet_b200_keyframe_destroy(kf);
-    return fail(ICET_B200_E_CUDA, std::string("keyframe copy: ") + cudaGetErrorString(e));
-  }
+  if (e != cudaSuccess) return fail(ICET_B200_E_CUDA, std::string("keyframe copy: ") + cudaGetErrorString(e));
   kf->n_gauss1 = *h_ng;
-  *out = kf;
+  *out = kf.release();
   return 0;
 }
 
@@ -609,7 +595,7 @@ int icet_b200_keyframe_create(icet_b200_ctx* c, const icet_b200_params* p, const
   rc = c->stage[0].ensure(std::max<size_t>(1, (size_t)3 * n1) * sizeof(float));
   if (rc) return rc;
   float* d_s1 = (float*)c->stage[0].p;
-  rc = upload_planes(c, d_s1, scan1, n1, ld1);
+  rc = upload_cloud(c, d_s1, scan1, n1, ld1);
   if (rc) return rc;
   return icet_b200_keyframe_create_device(c, p, d_s1, n1, n1, out);
 }
@@ -621,8 +607,6 @@ int icet_b200_keyframe_destroy(icet_b200_keyframe* kf) {
   cudaStreamSynchronize(c->stream);
   for (int l = 1; l < ICET_NLANE; l++)
     if (c->lanes[l]) cudaStreamSynchronize(c->lanes[l]);
-  kf->rec.release();
-  kf->vox.release();
   delete kf;
   return 0;
 }
@@ -643,30 +627,21 @@ int icet_b200_register_keyframe(icet_b200_keyframe* kf, const icet_b200_params* 
   CK(cudaEventSynchronize(c->ev_done[0]));
   rc = c->stage[0].ensure(std::max<size_t>(1, (size_t)3 * n2) * sizeof(float));
   if (rc) return rc;
-  rc = c->descbuf[0].ensure(sizeof(PairDesc));
-  if (rc) return rc;
   rc = c->x0buf[0].ensure(6 * sizeof(float));
   if (rc) return rc;
   rc = c->resbuf.ensure(sizeof(icet_b200_result));
   if (rc) return rc;
-  rc = ensure_pinned(c, 4096);
-  if (rc) return rc;
-  CK(cudaStreamSynchronize(c->stream));  // the pinned bounce buffer may still feed an earlier upload
   float* d_s2 = (float*)c->stage[0].p;
-  rc = upload_planes(c, d_s2, scan2, n2, ld2);
+  rc = upload_cloud(c, d_s2, scan2, n2, ld2);
   if (rc) return rc;
-  PairDesc* hd = (PairDesc*)c->pinned;
-  *hd = PairDesc{nullptr, d_s2, 0, 0, n2, n2};
-  CK(cudaMemcpyAsync(c->descbuf[0].p, hd, sizeof(PairDesc), cudaMemcpyHostToDevice, c->stream));
   const float* d_x0 = nullptr;
-  if (x0) {
-    float* hx = (float*)((char*)c->pinned + 256);
-    memcpy(hx, x0, 6 * sizeof(float));
-    CK(cudaMemcpyAsync(c->x0buf[0].p, hx, 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  if (x0) {  // (straight from the caller's array: the pinned bounce buffer is batch_device_impl's, which may grow it)
+    CK(cudaMemcpyAsync(c->x0buf[0].p, x0, 6 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
     d_x0 = (const float*)c->x0buf[0].p;
   }
+  const PairDesc desc{nullptr, d_s2, 0, 0, n2, n2};
   icet_b200_result* d_res = (icet_b200_result*)c->resbuf.p;
-  rc = run_chunk(c, p, 1, (const PairDesc*)c->descbuf[0].p, 0, n2, d_x0, d_res, false, 0, kf);
+  rc = batch_device_impl(c, p, 1, &desc, d_x0, d_res, false, nullptr, 0, kf);
   if (rc) return rc;
   CK(cudaMemcpyAsync(out, d_res, sizeof(icet_b200_result), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
@@ -677,17 +652,13 @@ int icet_b200_register_keyframe_batch_device(icet_b200_keyframe* kf, const icet_
                                              const float* const* scan2, const int32_t* n2, const float* x0,
                                              icet_b200_result* out) {
   int rc = keyframe_params(kf, p);
+  if (!rc) rc = check_pairs(npairs, false, nullptr, nullptr, scan2, n2, out);
   if (rc) return rc;
-  if (npairs < 0 || (npairs > 0 && (!scan2 || !n2 || !out))) return fail(ICET_B200_E_INVALID, "NULL argument");
   if (npairs == 0) return 0;
   icet_b200_ctx* c = kf->ctx;
   CK(cudaSetDevice(c->device));
   std::vector<PairDesc> d(npairs);
-  for (int i = 0; i < npairs; i++) {
-    if (n2[i] < 0 || (n2[i] > 0 && !scan2[i]))
-      return fail(ICET_B200_E_INVALID, "bad scan pointer / size in pair " + std::to_string(i));
-    d[i] = PairDesc{nullptr, scan2[i], 0, 0, n2[i], n2[i]};
-  }
+  for (int i = 0; i < npairs; i++) d[i] = PairDesc{nullptr, scan2[i], 0, 0, n2[i], n2[i]};
   return batch_device_impl(c, p, npairs, d.data(), x0, out, false, nullptr, 0, kf);
 }
 
