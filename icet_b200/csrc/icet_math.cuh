@@ -550,62 +550,14 @@ __device__ __forceinline__ bool masked_inv3(const double M[9], int mask, double 
   const double c11 = a * f - c * c, c12 = b * c - a * e, c22 = a * d - b * b;
   const double id = 1.0 / det;
   const double tr = a + d + f;
-  const double tri = (c00 + c11 + c22) * id;
-  if (!(tr * tri < 1e5)) return false;
+  const double csum = c00 + c11 + c22;
+  const double tri = csum * id;
+  // csum = l1 l2 + l1 l3 + l2 l3 >= tr^2 / 9e5 whenever cond < 1e5.  Below that it is rounding noise (M of rank one:
+  // every 2x2 minor vanishes), det is as well, and their ratio can pass the trace bound while M is singular.
+  if (!(tr * tri < 1e5) || !(csum > 1e-6 * (tr * tr))) return false;
   W[0] = c00 * id; W[1] = c01 * id; W[2] = c02 * id;
   W[3] = c01 * id; W[4] = c11 * id; W[5] = c12 * id;
   W[6] = c02 * id; W[7] = c12 * id; W[8] = c22 * id;
-  return true;
-}
-
-// Cholesky-based inverse of a symmetric 6x6 (row-major).  Returns false if not positive definite.
-// Every loop has compile-time bounds and is fully unrolled so that G / Gi live in registers
-// (the routine runs on ONE thread per pair and sits on the critical path of every iteration).
-__device__ __forceinline__ bool chol_inv6(const double* __restrict__ A, double* __restrict__ Ainv) {
-  double G[36];
-  bool ok = true;
-#pragma unroll
-  for (int j = 0; j < 6; j++) {
-    double s = A[j * 6 + j];
-#pragma unroll
-    for (int k = 0; k < j; k++) s -= G[j * 6 + k] * G[j * 6 + k];
-    ok = ok && (s > 0.0);
-    const double g = sqrt(s);
-    const double ig = 1.0 / g;
-    G[j * 6 + j] = g;
-#pragma unroll
-    for (int i = j + 1; i < 6; i++) {
-      double t = A[i * 6 + j];
-#pragma unroll
-      for (int k = 0; k < j; k++) t -= G[i * 6 + k] * G[j * 6 + k];
-      G[i * 6 + j] = t * ig;
-    }
-  }
-  if (!ok) return false;
-  // Gi = G^-1 (lower triangular)
-  double Gi[36];
-#pragma unroll
-  for (int j = 0; j < 6; j++) {
-    Gi[j * 6 + j] = 1.0 / G[j * 6 + j];
-#pragma unroll
-    for (int i = j + 1; i < 6; i++) {
-      double t = 0.0;
-#pragma unroll
-      for (int k = j; k < i; k++) t -= G[i * 6 + k] * Gi[k * 6 + j];
-      Gi[i * 6 + j] = t / G[i * 6 + i];
-    }
-  }
-  // Ainv = Gi^T Gi
-#pragma unroll
-  for (int i = 0; i < 6; i++)
-#pragma unroll
-    for (int j = 0; j <= i; j++) {
-      double t = 0.0;
-#pragma unroll
-      for (int k = i; k < 6; k++) t += Gi[k * 6 + i] * Gi[k * 6 + j];
-      Ainv[i * 6 + j] = t;
-      Ainv[j * 6 + i] = t;
-    }
   return true;
 }
 
@@ -614,7 +566,7 @@ __device__ __forceinline__ bool chol_inv6(const double* __restrict__ A, double* 
 // at reference src/icet.cpp:455-458 (only eigenvalues and sign-independent combinations of the
 // eigenvectors reach X; see DESIGN.md for the :479 inflation term).
 // All matrix indices are compile-time constants after unrolling, so A and U live in registers;
-// the routine is kept out of line because it runs only when the cheap condition bound fails.
+// the routine is kept out of line because it runs only when the warp solve's condition bound fails.
 __device__ __noinline__ void jacobi6(const double* __restrict__ Ain, double* __restrict__ ev_out,
                                      double* __restrict__ U_out) {
   double A[36], U[36];

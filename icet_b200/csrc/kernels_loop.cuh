@@ -314,8 +314,9 @@ __device__ __forceinline__ void vox_contrib(const Chunk& ck, int pair, int cell,
 }
 
 // ----------------------------------------------------------------------------------------------
-// K6: one thread per pair: Q = pinv(H^T W H), pred_stds, checkCondition, dx, X += dx (src/icet.cpp:410-433,
-// :443-492) and the transform / get_H trigonometry of the next iteration.  tot = the 28 sums over the voxels.
+// K6: Q = pinv(H^T W H), pred_stds, checkCondition, dx, X += dx (src/icet.cpp:410-433, :443-492) and the transform /
+// get_H trigonometry of the next iteration.  tot = the 28 sums over the voxels.  Every loop form runs the same
+// arithmetic: solve_pair_warp on one warp, and solve_pair on one lane of it when the warp form declines.
 // ----------------------------------------------------------------------------------------------
 // Odometry chaining (odometry.cpp:82 `X0 << X[0], ...`): the registration of pair k+1 starts from the solution of
 // pair k.  Called by the thread that has just written X / TR / J of `pair` in the LAST iteration, before that
@@ -362,6 +363,7 @@ __device__ __forceinline__ void mode_after_solve(const Chunk& ck, int pair, cons
   }
 }
 
+// solve_pair: the general case, one thread (eigen-decomposition + the reference's truncation loop).
 __device__ __noinline__ void solve_pair(const Chunk& ck, int pair, int iter, const double* tot, const ModeNow* cur = nullptr) {
   float* X = ck.X + pair * 6;
   double A[36], b[6];
@@ -382,68 +384,45 @@ __device__ __noinline__ void solve_pair(const Chunk& ck, int pair, int iter, con
   double Q[36], dx[6], stds[6];
   int dropped = 0, status = 0;
   double cond_out = 0.0;
-  bool fast = false;
-  if (!(ck.flags & ICET_B200_FLAG_FULL_EIG) && icet::chol_inv6(A, Q)) {
-    double trA = 0.0, trQ = 0.0;
-#pragma unroll
-    for (int k = 0; k < 6; k++) { trA += A[k * 6 + k]; trQ += Q[k * 6 + k]; }
-    // cond <= trace(A) * trace(A^-1); comfortably below the 1e6 cutoff => no axis is dropped and
-    // pinv == inverse, so dx = A^-1 b  (src/icet.cpp:410-433 with an empty while-loop at :469)
-    if (trA * trQ < 0.999e6) {
-      fast = true;
-      cond_out = -(trA * trQ);
+  double ev[6], U[36];
+  icet::jacobi6(A, ev, U);
+  // noise_mat = pinv(H^T W H) (:410-411) from the eigen-decomposition, with the rank rule of the COD
+  // (pivot > FLT_EPSILON * 6 * largest pivot) applied to the spectrum
+  {
+    double lm = 0.0;
+    for (int k = 0; k < 6; k++) lm = fmax(lm, fabs(ev[k]));
+    const double thr = (double)FLT_EPSILON * 6.0 * lm;
+    for (int i = 0; i < 36; i++) Q[i] = 0.0;
+    for (int k = 0; k < 6; k++) {
+      if (!(fabs(ev[k]) > thr)) continue;
+      const double il = 1.0 / ev[k];
+      for (int i = 0; i < 6; i++)
+        for (int j = 0; j < 6; j++) Q[i * 6 + j] += U[i * 6 + k] * U[j * 6 + k] * il;
     }
   }
-  if (fast) {
-#pragma unroll
-    for (int k = 0; k < 6; k++) {
-      double s = 0.0;
-#pragma unroll
-      for (int j = 0; j < 6; j++) s += Q[k * 6 + j] * b[j];
-      dx[k] = s;
-      stds[k] = sqrt(fabs(Q[k * 6 + k]));
-    }
-  } else {
-    double ev[6], U[36];
-    icet::jacobi6(A, ev, U);
-    // noise_mat = pinv(H^T W H) (:410-411) from the eigen-decomposition, with the rank rule of the COD
-    // (pivot > FLT_EPSILON * 6 * largest pivot) applied to the spectrum
-    {
-      double lm = 0.0;
-      for (int k = 0; k < 6; k++) lm = fmax(lm, fabs(ev[k]));
-      const double thr = (double)FLT_EPSILON * 6.0 * lm;
-      for (int i = 0; i < 36; i++) Q[i] = 0.0;
-      for (int k = 0; k < 6; k++) {
-        if (!(fabs(ev[k]) > thr)) continue;
-        const double il = 1.0 / ev[k];
-        for (int i = 0; i < 6; i++)
-          for (int j = 0; j < 6; j++) Q[i * 6 + j] += U[i * 6 + k] * U[j * 6 + k] * il;
-      }
-    }
-    for (int k = 0; k < 6; k++) stds[k] = sqrt(fabs(Q[k * 6 + k]));
-    const double cutoff = 1e6;
-    double condition = ev[5] / ev[0];
-    cond_out = condition;
-    int eyecount = 1;
-    while (fabs(condition) > cutoff) {  // checkCondition :469-486
-      if (eyecount > 5) { status = ICET_B200_COND_OVERFLOW; break; }
-      for (int k = 0; k < 6; k++) stds[k] += U[k * 6 + (eyecount - 1)];  // :479
-      dropped++;
-      condition = ev[5] / ev[eyecount];
-      eyecount++;
-    }
-    // dx = pinv(L2 lam U2^T) L2 U2^T b = sum over kept k of u_k (u_k . b) / lam_k, with the rank
-    // rule of the COD applied to the kept spectrum (:427-430)
-    double lmax = 0.0;
-    for (int k = dropped; k < 6; k++) lmax = fmax(lmax, fabs(ev[k]));
-    const double tiny = (double)FLT_EPSILON * (double)(6 - dropped) * lmax;
-    for (int k = 0; k < 6; k++) dx[k] = 0.0;
-    for (int k = dropped; k < 6; k++) {
-      if (!(fabs(ev[k]) > tiny)) continue;
-      double ub = 0.0;
-      for (int j = 0; j < 6; j++) ub += U[j * 6 + k] * b[j];
-      for (int j = 0; j < 6; j++) dx[j] += U[j * 6 + k] * (ub / ev[k]);
-    }
+  for (int k = 0; k < 6; k++) stds[k] = sqrt(fabs(Q[k * 6 + k]));
+  const double cutoff = 1e6;
+  double condition = ev[5] / ev[0];
+  cond_out = condition;
+  int eyecount = 1;
+  while (fabs(condition) > cutoff) {  // checkCondition :469-486
+    if (eyecount > 5) { status = ICET_B200_COND_OVERFLOW; break; }
+    for (int k = 0; k < 6; k++) stds[k] += U[k * 6 + (eyecount - 1)];  // :479
+    dropped++;
+    condition = ev[5] / ev[eyecount];
+    eyecount++;
+  }
+  // dx = pinv(L2 lam U2^T) L2 U2^T b = sum over kept k of u_k (u_k . b) / lam_k, with the rank
+  // rule of the COD applied to the kept spectrum (:427-430)
+  double lmax = 0.0;
+  for (int k = dropped; k < 6; k++) lmax = fmax(lmax, fabs(ev[k]));
+  const double tiny = (double)FLT_EPSILON * (double)(6 - dropped) * lmax;
+  for (int k = 0; k < 6; k++) dx[k] = 0.0;
+  for (int k = dropped; k < 6; k++) {
+    if (!(fabs(ev[k]) > tiny)) continue;
+    double ub = 0.0;
+    for (int j = 0; j < 6; j++) ub += U[j * 6 + k] * b[j];
+    for (int j = 0; j < 6; j++) dx[j] += U[j * 6 + k] * (ub / ev[k]);
   }
   float Xn[6];
   for (int k = 0; k < 6; k++) Xn[k] = (float)((double)__ldcg(X + k) + dx[k]);  // X += dx (:433), X is fp32
@@ -941,14 +920,17 @@ __global__ void __launch_bounds__(SOLVE_THREADS) k_solve6(const Chunk ck, int it
     s_tot[lane] = mine;
   }
   __syncwarp();
-  // (one thread: this kernel is bound by instruction fetch of once-executed code, the warp-parallel solve of
-  // k_loop is not faster here)
-  if (lane == 0) {
-    solve_pair(ck, pair, iter, s_tot);
-    s_rebuild = 0;
-    if (loop_incremental(ck) && iter < ck.runlen - 1) {
-      s_rebuild = ck.pm[pair].rebuild;  // (written by this thread a moment ago)
-      for (int k = 0; k < 12; k++) s_trb[k] = ck.pm[pair].TRb[k];
+  // warp 0: the solve of the cluster loop and k_loop, so that a batch row equals its single call byte for byte
+  if (threadIdx.x < 32) {
+    bool done = false;
+    if (!(ck.flags & ICET_B200_FLAG_FULL_EIG)) done = solve_pair_warp(ck, pair, iter, s_tot);
+    if (!done && lane == 0) solve_pair(ck, pair, iter, s_tot);
+    if (lane == 0) {
+      s_rebuild = 0;
+      if (loop_incremental(ck) && iter < ck.runlen - 1) {
+        s_rebuild = ck.pm[pair].rebuild;  // (written by this thread a moment ago)
+        for (int k = 0; k < 12; k++) s_trb[k] = ck.pm[pair].TRb[k];
+      }
     }
   }
   __syncthreads();
